@@ -8,6 +8,7 @@ suffstat update (-> one all-reduce of the suffstat deltas when N > 1).
   python bench.py --gpus 1 --steps 5 --warmup 3
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      # the CPU path, all host threads
+  python bench.py ... --dump-outputs DIR    # + what the last timed step computed, as DIR/<config>_<name>.npy
 
 Prints ONE JSON line (rank 0).  The headline keys (value, ms_per_step, roofline, e2e, cpu_baseline) are those of
 --workload (default C2, BASELINE.json configs[1], at every N so that the per-N values are comparable).  The same
@@ -33,6 +34,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 METRIC = "row_x_group_x_feature_scores_per_sec"
 UNIT = "scores/s"
@@ -89,27 +91,35 @@ class ClockSampler(object):
         self.proc = None
 
     def start(self):
+        """starts sampling, or resumes it after pause(): the rows of every sampling stretch are summarised together"""
         try:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.index), "--query-gpu=" + self.Q,
                                           "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
-            self.thread = threading.Thread(target=self._read, daemon=True)
+            self.thread = threading.Thread(target=self._read, args=(self.proc,), daemon=True)
             self.thread.start()
         except Exception:
             self.proc = None
 
-    def _read(self):
-        for line in self.proc.stdout:
+    def _read(self, proc):
+        for line in proc.stdout:
             self.rows.append([c.strip() for c in line.split(",")])
 
-    def stop(self):
+    def pause(self):
+        """ends the running sampler; its rows are kept"""
         if not self.proc:
-            return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
+            return
         self.proc.terminate()
         try:
             self.proc.wait(timeout=2)
         except Exception:
             self.proc.kill()
+        self.thread.join(timeout=2)
+
+    def stop(self):
+        if not self.proc and not self.rows:
+            return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
+        self.pause()
         sm, mx, reasons = [], [], set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         for r in self.rows:
@@ -296,8 +306,46 @@ def replica_check(st, device, n_total, world):
             "group_sizes_sum": int(round(float(t[:kmax].sum().item()))), "rows_total": int(n_total)}
 
 
+DUMP_BYTES = 60 << 20   # --dump-outputs writes at most this much in all (64 MB less room for the .npy headers)
+
+
+def dump_outputs(out_dir, tag, st, device, budget):
+    """Writes what the last timed step left for a caller of the sweep as out_dir/<tag>_<name>.npy, in at most `budget`
+    bytes: the group ids and sizes, every row's group id, a sample of the rows of the score matrix (of its last chunk of
+    rows where the step scored in chunks) and the resident suffstats.  Where an array does not fit, a sample of it is
+    written, drawn from a fixed seed: the same arguments give the same inputs and the same sample on every run, so two
+    builds can be compared array for array.  The score matrix is read through the library's own reader, which knows
+    the layout the step left it in; that is one host copy of the last chunk (a few GB at full size), untimed."""
+    t0 = time.perf_counter()
+    rng = np.random.default_rng(20_000)
+
+    def sample(n, cap):
+        return np.arange(n) if n <= cap else np.sort(rng.choice(n, max(1, int(cap)), replace=False))
+
+    groups = np.asarray(st.groups(), np.int64)
+    out = {"group_ids": groups.astype(np.float64),
+           "group_sizes": np.asarray([st.groupsize(int(g)) for g in groups], np.float64)}
+    left = budget - sum(a.nbytes for a in out.values())
+    a = st.assignments()
+    assert np.all(np.abs(a) < (1 << 24)), "group ids beyond the integers float32 holds exactly"
+    out["assignments"] = a[sample(a.size, left // 2 // 4)].astype(np.float32)
+    S = st.read_last_scores()
+    out["scores"] = S[sample(S.shape[0], left // 4 // (4 * max(1, S.shape[1])))].astype(np.float32)
+    del S
+    ptr, cnt = st.suffstat_buffer()
+    ss = np.empty(cnt, np.float64)
+    if cnt:
+        from common_b200 import dist as cbd
+        ss = cbd.as_tensor(ptr, cnt, device).cpu().numpy()
+    out["suffstats"] = ss[sample(cnt, left // 4 // 8)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, "%s_%s.npy" % (tag, name)), arr)
+    return {"shapes": {name: list(arr.shape) for name, arr in out.items()}, "seconds": time.perf_counter() - t0}
+
+
 def run_config(ctx, device, stream, comm, workload, args, rank, local_rank, world, scaling, peaks, want_e2e, want_parity,
-               want_kernels, want_cpu):
+               want_kernels, want_cpu, dump_budget=0):
     """one BASELINE.json configuration: data, state, warm-up, timed steps, (e2e), (parity), (per-kernel HBM records)"""
     import torch
     import torch.distributed as dist
@@ -361,6 +409,11 @@ def run_config(ctx, device, stream, comm, workload, args, rank, local_rank, worl
         for kk, v in st.last_timings(back).items():
             phase[kk] += v * steps / timed
     launches = ctx.launch_count() - launches0
+    dumped = None
+    if dump_budget and rank == 0:   # before any further sweep changes the state the last timed step left
+        clocks.pause()              # the sampler is to see the GPU under this load, not idle during the dump's copies
+        dumped = dump_outputs(args.dump_outputs, workload.upper() + ("_strong" if scaling == "strong" else ""), st, device,
+                              dump_budget)
     t = torch.tensor([ms_total], device=device, dtype=torch.float64)
     u = torch.tensor([float(units)], device=device, dtype=torch.float64)
     if world > 1:
@@ -373,6 +426,8 @@ def run_config(ctx, device, stream, comm, workload, args, rank, local_rank, worl
     extra = 0
     if ms_total < 1500.0:
         extra = int(min(4000, max(1, np.ceil((1500.0 - ms_total) / max(ms_total / steps, 1e-3)))))
+        if dumped is not None:
+            clocks.start()
         for j in range(extra):
             step(warmup + steps + j)
         barrier()
@@ -387,6 +442,8 @@ def run_config(ctx, device, stream, comm, workload, args, rank, local_rank, worl
            "scaling": scaling, "n_gpus": world, "rows_per_gpu": n, "rows_total": n_total, "groups": k, "features": D,
            "steps": steps, "warmup": warmup, "ms_per_step": ms_total / steps, "value": value, "unit": UNIT,
            "phase_ms_per_step": {kk: v / steps for kk, v in phase.items()}, "gpu_launches": int(launches), "clocks": clk}
+    if dumped:
+        rec["dumped_outputs"] = dumped
 
     # ---- replicas (N > 1): bit-identical suffstats on every rank, group sizes add up --------------------------------
     if world > 1:
@@ -575,7 +632,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of every configuration, write what its last timed step computed as "
+                         "DIR/<config>_<name>.npy (float32 / float64, %d MiB at most in all; rank 0)" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed: --impl b200 only")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -659,7 +723,8 @@ def main():
         is_head = (w == head and scal == "weak")
         rec = run_config(ctx, device, stream, comm, w, args, rank, local_rank, world, scal, peaks,
                          want_e2e=not args.no_e2e, want_parity=not args.no_parity, want_kernels=True,
-                         want_cpu=is_head and not args.no_cpu)
+                         want_cpu=is_head and not args.no_cpu,
+                         dump_budget=DUMP_BYTES // len(plan) if args.dump_outputs else 0)
         records.append(rec)
         import gc
         gc.collect()
