@@ -114,7 +114,9 @@ _PROTOS = {
     "msb_sample_discrete_log": (C.c_int, [_P, _P, _SZ, _SZ, _SZ, _P, _P]),
     "msb_philox_uniforms": (C.c_int, [_P, C.c_uint64, C.c_uint64, C.c_uint64, _SZ, _P]),
     "msb_selftest_expf": (C.c_int, [_P, _P, _SZ, _P]),
+    "msb_selftest_expf2": (C.c_int, [_P, C.POINTER(C.c_uint64)]),
     "msb_selftest_division": (C.c_int, [_P, C.c_uint64, _SZ, C.POINTER(C.c_uint64)]),
+    "msb_selftest_skip_rule": (C.c_int, [_P, _P, _P, _P, _SZ, _P]),
     "msb_state_sweep": (C.c_int, [_P, _SZ, _SZ, C.POINTER(SweepOpts), C.POINTER(SweepResult)]),
     "msb_state_sweep_wait": (C.c_int, [_P, C.POINTER(SweepResult)]),
     "msb_state_delta_buffer": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),

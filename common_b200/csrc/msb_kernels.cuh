@@ -977,26 +977,48 @@ __device__ __forceinline__ float div_markstein(float p, float acc, float y) {
   return __fmaf_rn(r, y, q0);
 }
 
+// the same sequence two quotients at a time (FMUL2 / FFMA2): the same roundings as div_markstein (a multiply feeding
+// an FFMA2 has nothing ptxas could contract it with)
+__device__ __forceinline__ float2 div_markstein2(float2 p, float acc, float y) {
+  const float2 y2 = make_float2(y, y);
+  const float2 q0 = __fmul2_rn(p, y2);
+  const float2 r = __ffma2_rn(make_float2(-acc, -acc), q0, p);
+  return __ffma2_rn(r, y2, q0);
+}
+
 // Sparsity: exp(s - max) underflows to exactly 0 below -104, which in a mixture is the case for most groups of
 // most rows.  A batch of eight groups whose p is exactly 0 in every lane of the warp leaves every live dart
 // unchanged (dart - 0), so it is skipped as a whole (dead8(k0), warp-uniform); the same test lets the exp pass
 // skip the polynomial (exp_is_zero).  Results are bit-identical, only the work drops.
 __device__ __forceinline__ bool exp_is_zero(float x) { return x < -104.0f; }  // false for NaN, like msb_expf
 
-// all 32 lanes of the warp must call this (lanes without a row pass found = true)
-template <typename F, typename G>
-__device__ __forceinline__ void dart_walk(int K, float acc, float dart, bool found, int &pick, F p_of, G dead8) {
+// The walk's exact skip (DESIGN.md section 4.3): a dart d >= 2^-60 stays bit for bit, and so makes no pick, over a batch
+// whose largest p has the biased exponent e (every p < 2^(e - 126)) when acc is in [1, 2^24] and e <= Ea + Ed - 154
+// (Ea, Ed: the biased exponents of acc and d): then every RN(p / acc) is below half the spacing of the floats just
+// below d.  e = 255 (a NaN p) never passes.
+__device__ __forceinline__ bool dart_keeps(uint32_t e, float acc, float d) {
+  return acc >= 1.0f && acc <= 16777216.0f && d >= 0x1p-60f &&
+         (int)e <= (__float_as_int(acc) >> 23) - 154 + (__float_as_int(d) >> 23);
+}
+
+// all 32 lanes of the warp must call this (lanes without a row pass found = true).
+// skip8(k0, found, dart): this lane's dart and pick provably stay as they are over the batch k0 .. k0 + 7; the batch
+// is skipped when that holds in every lane.  PADDED: p_of(k) is +0 for K <= k < K rounded up to 8.
+template <bool PADDED = false, typename F, typename G>
+__device__ __forceinline__ void dart_walk(int K, float acc, float dart, bool found, int &pick, F p_of, G skip8) {
   const float y = __frcp_rn(acc);
   const bool odd = !(acc >= 1.0f && acc <= 16777216.0f);
   pick = K - 1;
   for (int k0 = 0; k0 < K; k0 += 8) {
-    // every p of the batch is +0 in every lane: q = +0 and dart - 0 = dart, unless a lane sits exactly on dart <= 0
-    if (dead8(k0) && __all_sync(0xffffffffu, found || dart > 0.f)) continue;
+    if (__all_sync(0xffffffffu, skip8(k0, found, dart))) continue;
     float p[8], q[8];
 #pragma unroll
-    for (int j = 0; j < 8; j++) p[j] = k0 + j < K ? p_of(k0 + j) : 0.f;
+    for (int j = 0; j < 8; j++) p[j] = PADDED || k0 + j < K ? p_of(k0 + j) : 0.f;
 #pragma unroll
-    for (int j = 0; j < 8; j++) q[j] = div_markstein(p[j], acc, y);
+    for (int j = 0; j < 8; j += 2) {
+      const float2 qq = div_markstein2(make_float2(p[j], p[j + 1]), acc, y);
+      q[j] = qq.x; q[j + 1] = qq.y;
+    }
     const float dart0 = dart;
     const int pick0 = pick;
     const bool found0 = found;
@@ -1005,7 +1027,8 @@ __device__ __forceinline__ void dart_walk(int K, float acc, float dart, bool fou
     for (int j = 0; j < 8; j++) {
       suspect |= !found && dart < 0x1p-60f && p[j] < 0x1p-100f && p[j] > 0.f;
       dart = __fsub_rn(dart, q[j]);
-      if (!found && dart <= 0.f && k0 + j < K) { pick = k0 + j; found = true; }
+      // a padding element (p = +0) cannot make the pick: a dart not found before it is > 0 or NaN and stays so
+      if (!found && dart <= 0.f && (PADDED || k0 + j < K)) { pick = k0 + j; found = true; }
     }
     if (__any_sync(0xffffffffu, suspect)) {  // rare: redo the batch with the IEEE division
       dart = dart0; pick = pick0; found = found0;
@@ -1046,7 +1069,9 @@ __global__ void sample_kernel(const float *__restrict__ scores, size_t ld, int K
   float dart = 0.f;
   if (valid) dart = uniforms ? uniforms[i] : philox_u01(seed, row_id0 + i, sweep);
   int pick;
-  dart_walk(K, acc, dart, !valid, pick, [&](int k) { return msb_expf(__fsub_rn(s[k], m)); }, dead8);
+  // every p of a dead batch is +0 in every lane: q = +0 and dart - 0 = dart, unless a lane sits exactly on dart <= 0
+  dart_walk(K, acc, dart, !valid, pick, [&](int k) { return msb_expf(__fsub_rn(s[k], m)); },
+            [&](int k0, bool f, float d) { return dead8(k0) && (f || d > 0.f); });
   if (!valid) return;
   if (out_col) out_col[i] = pick;
   if (out_slot) out_slot[i] = col2slot ? col2slot[pick] : pick;
@@ -1112,7 +1137,8 @@ __global__ void sample_blocked_kernel(const float *__restrict__ scores, size_t l
     const uint64_t w = b < 64 ? l0 : (b < 128 ? l1 : (b < 192 ? l2 : l3));
     return !((w >> (b & 63)) & 1ull);
   };
-  dart_walk(K, acc, dart, !valid, pick, [&](int kk) { return msb_expf(__fsub_rn(s[(size_t)kk * 32], m)); }, dead8_known);
+  dart_walk(K, acc, dart, !valid, pick, [&](int kk) { return msb_expf(__fsub_rn(s[(size_t)kk * 32], m)); },
+            [&](int k0, bool f, float d) { return dead8_known(k0) && (f || d > 0.f); });
   if (!valid) return;
   if (out_col) out_col[i] = pick;
   if (out_slot) out_slot[i] = col2slot ? col2slot[pick] : pick;
@@ -1124,8 +1150,22 @@ __global__ void selftest_expf_kernel(const float *__restrict__ x, size_t n, floa
   if (i < n) y[i] = msb_expf(x[i]);
 }
 
+// msb_expf2_dense against msb_expf on every float of [-86, 0]: thread t takes the pair -f(2t), -f(2t + 1), where f(b)
+// is the float with the bits b (b = 0 is -0); the last thread takes -86 and +0.  Counts the differing results.
+constexpr uint32_t EXPF2_LAST_BITS = 0x42AC0000u;  // 86.0f (even)
+__global__ void selftest_expf2_kernel(unsigned long long *mismatches) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t > EXPF2_LAST_BITS / 2) return;
+  float2 x = make_float2(-__uint_as_float(2 * t), -__uint_as_float(2 * t + 1));
+  if (t == EXPF2_LAST_BITS / 2) x = make_float2(-86.0f, 0.0f);
+  const float2 y = msb_expf2_dense(x);
+  const unsigned bad = (__float_as_uint(y.x) != __float_as_uint(msb_expf(x.x))) +
+                       (__float_as_uint(y.y) != __float_as_uint(msb_expf(x.y)));
+  if (bad) atomicAdd(mismatches, (unsigned long long)bad);
+}
+
 // q[i] = (a[i] / b[i] by Markstein's sequence) != __fdiv_rn(a[i], b[i]) counted: device self-test of dart_walk's
-// division on pseudo-random operands p in [2^-100, 1], acc in [1, 2^24) (plus exact zeros)
+// division, scalar and packed, on pseudo-random operands p in [2^-100, 1], acc in [1, 2^24) (plus exact zeros)
 __global__ void selftest_division_kernel(uint64_t seed, size_t n, unsigned long long *mismatches) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -1138,9 +1178,24 @@ __global__ void selftest_division_kernel(uint64_t seed, size_t n, unsigned long 
   if ((r[3] & 63u) == 0) p = 0.f;
   const uint32_t ae = 127 + ((r[2] >> 8) % 24);
   const float acc = __uint_as_float((ae << 23) | (r[1] & 0x7fffffu));
-  const float got = div_markstein(p, acc, __frcp_rn(acc));
-  const float want = __fdiv_rn(p, acc);
-  if (__float_as_uint(got) != __float_as_uint(want)) atomicAdd(mismatches, 1ull);
+  // a second dividend for the packed form the walk uses: another mantissa and exponent from the same block
+  float p2 = __uint_as_float(((127 - ((r[3] >> 8) % 101)) << 23) | (r[3] >> 9));
+  if (p2 > 1.0f) p2 = 1.0f;
+  if ((r[3] & 0xFC0u) == 0) p2 = 0.f;
+  const float y = __frcp_rn(acc);
+  const float got = div_markstein(p, acc, y);
+  const float2 got2 = div_markstein2(make_float2(p, p2), acc, y);
+  const float want = __fdiv_rn(p, acc), want2 = __fdiv_rn(p2, acc);
+  const unsigned bad = (__float_as_uint(got) != __float_as_uint(want)) + (__float_as_uint(got2.x) != __float_as_uint(want)) +
+                       (__float_as_uint(got2.y) != __float_as_uint(want2));
+  if (bad) atomicAdd(mismatches, (unsigned long long)bad);
+}
+
+// out[i] = dart_keeps(e[i], acc[i], d[i]): the walk's skip test on given operands, for the exact check on the host
+__global__ void selftest_skip_rule_kernel(const uint8_t *__restrict__ e, const float *__restrict__ acc,
+                                          const float *__restrict__ d, size_t n, uint8_t *__restrict__ out) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = dart_keeps(e[i], acc[i], d[i]) ? 1 : 0;
 }
 
 // blocked -> row-major copy of a score matrix (diagnostics / tests)

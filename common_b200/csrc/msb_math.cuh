@@ -50,6 +50,33 @@ __device__ __forceinline__ float msb_expf(float x) {
   return x_in >= -104.0f ? y : (x_in != x_in ? x_in : 0.0f);
 }
 
+// msb_expf of two arguments that both lie in [-86, 0] (not NaN), with the packed fp32 instructions of sm_100
+// (FMUL2 / FADD2 / FFMA2: one issue slot per pair).  The same operations in the same order, so the same bits:
+//   * the clamp and the final select are identities on that range, and a - b is a + (-b) in IEEE arithmetic;
+//   * k = rint(x log2e) is in [-124, 0], so kk = max(k, -125) = k and the subnormal factor 2^(k - kk) is 1;
+//   * kbias = 1.5 * 2^23 + k has the bits 0x4B400000 + k, and 0x4B400000 << 23 is 0 mod 2^32, so adding
+//     kbias_bits << 23 to p's bits adds exactly k << 23 to its exponent field.
+// The one exception is the add of 1.5 * 2^23 to x log2e, kept as two scalar FADDs: ptxas contracts mul.rn.f32x2
+// followed by add.rn.f32x2 into one FFMA2 despite the rounding modifiers, and the fused form can round k differently.
+// Checked over every float of the range against msb_expf by msb_selftest_expf2.
+__device__ __forceinline__ float2 msb_expf2_dense(float2 x) {
+  const float2 xl = __fmul2_rn(x, make_float2(1.44269504f, 1.44269504f));
+  const float2 kbias = make_float2(__fadd_rn(xl.x, 12582912.0f), __fadd_rn(xl.y, 12582912.0f));
+  const float2 kf = __fadd2_rn(kbias, make_float2(-12582912.0f, -12582912.0f));
+  float2 r = __ffma2_rn(kf, make_float2(-0.693145752f, -0.693145752f), x);
+  r = __ffma2_rn(kf, make_float2(-1.42860677e-6f, -1.42860677e-6f), r);
+  float2 p = __ffma2_rn(make_float2(1.9875691500e-4f, 1.9875691500e-4f), r, make_float2(1.3981999507e-3f, 1.3981999507e-3f));
+  p = __ffma2_rn(p, r, make_float2(8.3334519073e-3f, 8.3334519073e-3f));
+  p = __ffma2_rn(p, r, make_float2(4.1665795894e-2f, 4.1665795894e-2f));
+  p = __ffma2_rn(p, r, make_float2(1.6666665459e-1f, 1.6666665459e-1f));
+  p = __ffma2_rn(p, r, make_float2(5.0000001201e-1f, 5.0000001201e-1f));
+  const float2 r2 = __fmul2_rn(r, r);
+  p = __ffma2_rn(p, r2, r);
+  p = __fadd2_rn(p, make_float2(1.0f, 1.0f));
+  return make_float2(__int_as_float(__float_as_int(p.x) + (__float_as_int(kbias.x) << 23)),
+                     __int_as_float(__float_as_int(p.y) + (__float_as_int(kbias.y) << 23)));
+}
+
 // ---------------------------------------------------------------------------
 // Philox4x32-10 (Salmon et al. SC'11).  key = seed, counter = (row, sweep).
 // ---------------------------------------------------------------------------

@@ -133,17 +133,53 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t
 // ---------------------------------------------------------------------------------------------------
 // ROWMAJOR: the scores are row-major [row][ld] (the NIW kernels accumulate into that layout): the tile is filled
 // by coalesced loads (lane = group) and stored transposed with pitch 33, conflict-free both ways.
+// rowmax (may be null): the row maxima the score kernel's epilogue left (ordered integers, 0x80808080 where none was
+// written); pass 1 then runs only for a warp with such a row.
+//
+// Shared memory per warp: the tile, K rounded up to 8 groups (pass 2 writes p = +0 into the padding, so the walk reads
+// whole batches unconditionally), then one byte per (batch, lane): the biased exponent of the batch's largest p.
+// Layout [WARPS tiles][WARPS mbarriers][WARPS exponent arrays]; sample_tile_smem() gives the size.
+__host__ __device__ inline uint32_t sample_tile_bytes(int K, bool rowmajor) {
+  return ((uint32_t)(K + 7) / 8u * 8u * (rowmajor ? 33u : 32u) * 4u + 127u) / 128u * 128u;
+}
+__host__ __device__ inline size_t sample_tile_smem(int warps, int K, bool rowmajor) {
+  return (size_t)warps * (sample_tile_bytes(K, rowmajor) + sizeof(uint64_t) + (size_t)(K + 7) / 8 * 32) + 64;
+}
+
+// 3-input minimum / maximum (sm_100) that return NaN when an input is NaN
+__device__ __forceinline__ float fmin3_nan(float a, float b, float c) {
+  float d;
+  asm("min.NaN.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
+  return d;
+}
+__device__ __forceinline__ float fmax3_nan(float a, float b, float c) {
+  float d;
+  asm("max.NaN.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
+  return d;
+}
+__device__ __forceinline__ float fmax8_nan(const float *v) {
+  return fmax3_nan(fmax3_nan(v[0], v[1], v[2]), fmax3_nan(v[3], v[4], v[5]), fmax3_nan(v[6], v[7], v[7]));
+}
+__device__ __forceinline__ float fmin8_nan(const float *v) {
+  return fmin3_nan(fmin3_nan(v[0], v[1], v[2]), fmin3_nan(v[3], v[4], v[5]), fmin3_nan(v[6], v[7], v[7]));
+}
+
 template <int WARPS, bool ROWMAJOR>
 __global__ void __launch_bounds__(WARPS * 32)
 sample_tile_kernel(const float *__restrict__ scores, size_t ld, size_t skip, int K, size_t nrows,
                    const float *__restrict__ uniforms, uint64_t seed, uint64_t sweep, uint64_t row_id0,
-                   const int32_t *__restrict__ col2slot, int32_t *__restrict__ out_col, int32_t *__restrict__ out_slot) {
+                   const int32_t *__restrict__ col2slot, int32_t *__restrict__ out_col, int32_t *__restrict__ out_slot,
+                   const int *__restrict__ rowmax) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   constexpr int P = ROWMAJOR ? 33 : 32;  // tile pitch in floats: element (group k, row r) at tile[k * P + r]
-  const uint32_t tile_bytes = ((uint32_t)K * P * 4u + 127u) / 128u * 128u;
+  const uint32_t tile_bytes = sample_tile_bytes(K, ROWMAJOR);
+  const uint32_t copy_bytes = (uint32_t)K * 128u;   // the blocked layout's [K][32] tile
+  const int nb = (K + 7) / 8;                        // batches of eight groups
   float *tile = reinterpret_cast<float *>(smem_raw + (size_t)warp * tile_bytes);
   uint64_t *bar = reinterpret_cast<uint64_t *>(smem_raw + (size_t)WARPS * tile_bytes) + warp;
+  uint8_t *pexp = reinterpret_cast<uint8_t *>(smem_raw + (size_t)WARPS * (tile_bytes + sizeof(uint64_t))) +
+                  (size_t)warp * nb * 32 + lane;
   if (lane == 0) {
     mbar_init(smem_u32(bar), 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -163,8 +199,8 @@ sample_tile_kernel(const float *__restrict__ scores, size_t ld, size_t skip, int
       __syncwarp();
     } else {
       if (lane == 0) {
-        mbar_expect_tx(smem_u32(bar), tile_bytes);
-        bulk_g2s(smem_u32(tile), scores + blk * ld * 32, tile_bytes, smem_u32(bar));
+        mbar_expect_tx(smem_u32(bar), copy_bytes);
+        bulk_g2s(smem_u32(tile), scores + blk * ld * 32, copy_bytes, smem_u32(bar));
       }
       mbar_wait(smem_u32(bar), parity);
       parity ^= 1u;
@@ -172,62 +208,86 @@ sample_tile_kernel(const float *__restrict__ scores, size_t ld, size_t skip, int
     const long long i = (long long)(blk * 32 + lane) - (long long)skip;  // row of this lane, relative to the first valid row
     const bool valid = i >= 0 && (size_t)i < nrows;
     float *s = tile + lane;
-    // pass 1: max (exact and order-independent: four partial maxima for instruction-level parallelism)
-    float m0 = s[0], m1 = m0, m2 = m0, m3 = m0, lo0 = m0, lo1 = m0;
-    int k = 1;
-    for (; k + 3 < K; k += 4) {
-      const float a0 = s[k * P], a1 = s[(k + 1) * P], a2 = s[(k + 2) * P], a3 = s[(k + 3) * P];
-      m0 = fmaxf(m0, a0); m1 = fmaxf(m1, a1); m2 = fmaxf(m2, a2); m3 = fmaxf(m3, a3);
-      lo0 = fminf(lo0, fminf(a0, a1)); lo1 = fminf(lo1, fminf(a2, a3));
+    // pass 1: max (exact and order-independent: four partial maxima for instruction-level parallelism), unless the
+    // score kernel left it: the same floats, the same maximum
+    float m = 0.f;
+    bool scan = true;
+    if (rowmax) {
+      const int ord = rowmax[blk * 32 + lane];
+      scan = ord == (int)0x80808080;
+      m = ordered_float(ord);
     }
-    for (; k < K; k++) { m0 = fmaxf(m0, s[k * P]); lo0 = fminf(lo0, s[k * P]); }
-    const float m = fmaxf(fmaxf(m0, m1), fmaxf(m2, m3));
-    // A row whose smallest score is still within exp's range keeps every batch of eight groups alive: the
-    // batch-skipping passes below would only add their votes.  Then take the dense passes (same results).
-    const bool dense = __any_sync(0xffffffffu, valid && !exp_is_zero(__fsub_rn(fminf(lo0, lo1), m)));
-    // pass 2: p = exp(s - m) (independent per k, kept in the tile) and the in-order double sum (the only chain)
-    // Batches of eight groups whose exp underflows to 0 in every lane are only recorded (bit kb of `live`):
-    // nothing to add to the sum, nothing to store, and the walk below skips them too (K <= 512 here).
+    if (__any_sync(0xffffffffu, scan)) {
+      float m0 = s[0], m1 = m0, m2 = m0, m3 = m0;
+      int k = 1;
+      for (; k + 3 < K; k += 4) {
+        m0 = fmaxf(m0, s[k * P]); m1 = fmaxf(m1, s[(k + 1) * P]);
+        m2 = fmaxf(m2, s[(k + 2) * P]); m3 = fmaxf(m3, s[(k + 3) * P]);
+      }
+      for (; k < K; k++) m0 = fmaxf(m0, s[k * P]);
+      if (scan) m = fmaxf(fmaxf(m0, m1), fmaxf(m2, m3));
+    }
+    // pass 2: p = exp(s - m) (independent per k, kept in the tile) and the in-order double sum (the only chain),
+    // a batch of eight groups at a time, chosen by a warp vote on its x = s - m:
+    //   dead   every x < -104: every p is +0 (nothing to add to the sum, +0 stored)
+    //   fast   every x in [-86, 0]: msb_expf2_dense, two groups per instruction (the same bits)
+    //   else   msb_expf one group at a time (NaN, -inf, subnormal results)
+    // and the biased exponent of the batch's largest p is recorded for the walk (NaN gives 255).
     double acc_d = 0.0;
-    uint64_t live = 0;
-    if (dense) {
-      live = ~0ull;
-#pragma unroll 8
-      for (k = 0; k < K; k++) {
-        const float p = msb_expf(__fsub_rn(s[k * P], m));
-        s[k * P] = p;
-        acc_d = __dadd_rn(acc_d, (double)p);
-      }
-    } else
-    for (int k0 = 0; k0 < K; k0 += 8) {
-      float x[8];
-      bool any = false;
+    const float2 nm = make_float2(-m, -m);
+    auto batch = [&](int k0, auto tail_tag) {
+      constexpr bool TAIL = decltype(tail_tag)::value;
+      float x[8], p[8];
 #pragma unroll
-      for (int j = 0; j < 8; j++) {
-        x[j] = k0 + j < K ? __fsub_rn(s[(k0 + j) * P], m) : -CUDART_INF_F;
-        any |= !exp_is_zero(x[j]);
+      for (int j = 0; j < 8; j += 2) {  // s - m as s + (-m): the same rounding
+        const float2 x2 = __fadd2_rn(make_float2(s[(k0 + j) * P], s[(k0 + j + 1) * P]), nm);
+        x[j] = x2.x; x[j + 1] = x2.y;
       }
-      if (!__any_sync(0xffffffffu, any)) continue;
-      live |= 1ull << (k0 >> 3);
+      if constexpr (TAIL) {
 #pragma unroll
-      for (int j = 0; j < 8; j++) {
-        if (k0 + j < K) {
-          const float p = msb_expf(x[j]);
-          s[(k0 + j) * P] = p;
-          acc_d = __dadd_rn(acc_d, (double)p);
+        for (int j = 0; j < 8; j++) if (k0 + j >= K) x[j] = -CUDART_INF_F;
+      }
+      const float xhi = fmax8_nan(x);
+      if (__all_sync(0xffffffffu, xhi < -104.0f)) {
+#pragma unroll
+        for (int j = 0; j < 8; j++) s[(k0 + j) * P] = 0.f;
+        pexp[(k0 >> 3) * 32] = 0;
+        return;
+      }
+      const float xlo = fmin8_nan(x);
+      if (__all_sync(0xffffffffu, xlo >= -86.0f && xhi <= 0.0f)) {
+#pragma unroll
+        for (int j = 0; j < 8; j += 2) {
+          const float2 p2 = msb_expf2_dense(make_float2(x[j], x[j + 1]));
+          p[j] = p2.x; p[j + 1] = p2.y;
         }
+      } else {
+#pragma unroll
+        for (int j = 0; j < 8; j++) p[j] = msb_expf(x[j]);
       }
-    }
+#pragma unroll
+      for (int j = 0; j < 8; j++) {
+        s[(k0 + j) * P] = p[j];
+        if (!TAIL || k0 + j < K) acc_d = __dadd_rn(acc_d, (double)p[j]);
+      }
+      pexp[(k0 >> 3) * 32] = (uint8_t)(__float_as_uint(fmax8_nan(p)) >> 23);
+    };
+    const int kfull = K & ~7;
+    for (int k0 = 0; k0 < kfull; k0 += 8) batch(k0, std::false_type{});
+    if (kfull < K) batch(kfull, std::true_type{});
     const float acc = __double2float_rn(acc_d);
     float dart = 0.f;
     if (valid) dart = uniforms ? uniforms[i] : philox_u01(seed, row_id0 + (uint64_t)i, sweep);
-    // pass 3: the dart walk (msb_kernels.cuh), quotients from the tile
+    // pass 3: the dart walk (msb_kernels.cuh), quotients from the tile.  A lane whose dart d >= 2^-60 is normal keeps
+    // d bit for bit over a batch whose every q = RN(p / acc) is below h = 2^(floor(log2 d) - 25) -- at most half the
+    // spacing of the floats just below d, so RN(d - q) = d -- and then makes no pick either (d stays > 0).  With
+    // E the batch's recorded exponent (every p < 2^(E - 126)) and acc in [1, 2^24] (acc >= 2^(Ea - 127)),
+    //   E <= Ea + Ed - 154  gives  p / acc < 2^(Ed - 153) = h / 2,  so  RN(p / acc) <= pred(h) < h
+    // (Ea, Ed: biased exponents of acc and d; E = 255 for a NaN p never passes).  Such a batch is skipped when every
+    // lane still walking passes; the exact conditions are in DESIGN.md section 4.3.
     int pick;
-    if (dense)
-      dart_walk(K, acc, dart, !valid, pick, [&](int kk) { return s[kk * P]; }, [](int) { return false; });
-    else
-      dart_walk(K, acc, dart, !valid, pick, [&](int kk) { return ((live >> (kk >> 3)) & 1ull) ? s[kk * P] : 0.f; },
-                [&](int k0) { return !((live >> (k0 >> 3)) & 1ull); });
+    dart_walk<true>(K, acc, dart, !valid, pick, [&](int kk) { return s[kk * P]; },
+                    [&](int k0, bool f, float d) { return f || dart_keeps(pexp[(k0 >> 3) * 32], acc, d); });
     if (valid) {
       if (out_col) out_col[i] = pick;
       if (out_slot) out_slot[i] = col2slot ? col2slot[pick] : pick;
@@ -259,7 +319,8 @@ __global__ void __launch_bounds__(NW * 32, 1)
 score_kernel(const FeatDev *__restrict__ feats, int nfeat, const float *__restrict__ params, size_t region_rows,
              uint32_t stage_bytes, int S, const float *__restrict__ base, float *__restrict__ scores, size_t ld,
              size_t row_org, size_t row_lo, size_t row_hi, const double *__restrict__ hp,
-             const double *__restrict__ ss, const int32_t *__restrict__ col2slot, int ncols, int ktiles, int tail_g) {
+             const double *__restrict__ ss, const int32_t *__restrict__ col2slot, int ncols, int ktiles, int tail_g,
+             int *__restrict__ rowmax) {
   constexpr int KT = 32 * V;
   constexpr int RL = RW / 32;
   constexpr int RB = NW * RW;                                   // rows per block
@@ -570,8 +631,14 @@ score_kernel(const FeatDev *__restrict__ feats, int nfeat, const float *__restri
           const size_t rb = (row0 - row_org) / 32 + j;
           if (row0 + (size_t)j * 32 < row_hi) {
             float *dst = scores + (rb * ld + (size_t)kt * KT) * 32 + lane;
+            float mx = -CUDART_INF_F;
 #pragma unroll
-            for (int c = 0; c < G; c++) dst[(size_t)c * 32] = tile[lane * (KT + 1) + c];
+            for (int c = 0; c < G; c++) {
+              const float v = tile[lane * (KT + 1) + c];
+              dst[(size_t)c * 32] = v;
+              if (kt * KT + c < ncols) mx = fmaxf(mx, v);
+            }
+            if (rowmax) atomicMax(rowmax + rb * 32 + lane, float_ordered(mx));
           }
         }
       }
@@ -609,8 +676,15 @@ score_kernel(const FeatDev *__restrict__ feats, int nfeat, const float *__restri
       const size_t rb = (row0 - row_org) / 32 + j;
       if (row0 + (size_t)j * 32 < row_hi) {
         float *dst = scores + (rb * ld + (size_t)kt * KT) * 32 + lane;
+        // the row's largest score over this k-tile's real groups goes to the sampler, as in score_bundle_kernel
+        float mx = -CUDART_INF_F;
 #pragma unroll 8
-        for (int c = 0; c < KT; c++) dst[(size_t)c * 32] = tile[lane * (KT + 1) + c];
+        for (int c = 0; c < KT; c++) {
+          const float v = tile[lane * (KT + 1) + c];
+          dst[(size_t)c * 32] = v;
+          if (kt * KT + c < ncols) mx = fmaxf(mx, v);
+        }
+        if (rowmax) atomicMax(rowmax + rb * 32 + lane, float_ordered(mx));
       }
     }
   }

@@ -1540,6 +1540,22 @@ static int launch_score(msb_state *st, size_t row_lo, size_t row_hi, float *scor
     const size_t grid = (size_t)cdiv(nrows, RB) * ktiles;
     if (grid >= (1ull << 31)) return fail(MSB_ERR_UNSUPPORTED, "score grid too large: sweep a smaller row range");
     static const bool no_bundle = getenv("MSB_NO_BUNDLE") != nullptr;
+    const bool persistent = getenv("MSB_PERSISTENT") != nullptr;   // read per call: the test switches it
+    // The sweep's sampler takes the row maxima from the blocked epilogues of score_bundle_kernel and score_kernel when
+    // nothing is added to the matrix afterwards (NIW, dm).  The persistent tables-only kernel stores straight from
+    // registers, where a lane holds one group of 32 rows rather than one row, and does not emit them.
+    int *rowmax = nullptr;
+    if (want_rowmax && blocked && !st->has_niw && !st->has_dm && !(st->tables_only && persistent) && !getenv("MSB_NO_ROWMAX")) {
+      const size_t need = nrows + 128;
+      if (st->rowmax_cap < need) {
+        CU_TRY(cudaFree(st->d_rowmax)); st->d_rowmax = nullptr; st->rowmax_cap = 0;
+        CU_TRY(cudaMalloc(&st->d_rowmax, need * sizeof(int)));
+        st->rowmax_cap = need;
+      }
+      CU_TRY(cudaMemsetAsync(st->d_rowmax, 0x80, need * sizeof(int), ctx->stream));   // below every finite float in the ordered encoding
+      rowmax = st->d_rowmax;
+      st->rowmax_valid = true;
+    }
     if (!st->tables_only && !no_bundle && (st->cfg == 1 || st->cfg == 2 || st->cfg == 4)) {
       // General kernel, bundled ring (score_bundle_kernel): three stages of a third of the shared memory each, every
       // stage filled with as many consecutive features of the walk order as fit.
@@ -1590,19 +1606,6 @@ static int launch_score(msb_state *st, size_t row_lo, size_t row_hi, float *scor
           if (blocked) LAUNCH(ctx, (score_bundle_kernel<V_, RW_, NW_, true>), (unsigned)grid, NW_ * 32, smem_b, MSB_BUNDLE_ARGS); \
           else LAUNCH(ctx, (score_bundle_kernel<V_, RW_, NW_, false>), (unsigned)grid, NW_ * 32, smem_b, MSB_BUNDLE_ARGS);        \
         } while (0)
-        // the sweep's sampler takes the row maxima from this kernel's epilogue when nothing is added to the matrix afterwards
-        int *rowmax = nullptr;
-        if (want_rowmax && blocked && !st->has_niw && !st->has_dm && !getenv("MSB_NO_ROWMAX")) {
-          const size_t need = nrows + 128;
-          if (st->rowmax_cap < need) {
-            CU_TRY(cudaFree(st->d_rowmax)); st->d_rowmax = nullptr; st->rowmax_cap = 0;
-            CU_TRY(cudaMalloc(&st->d_rowmax, need * sizeof(int)));
-            st->rowmax_cap = need;
-          }
-          CU_TRY(cudaMemsetAsync(st->d_rowmax, 0x80, need * sizeof(int), ctx->stream));   // below every finite float in the ordered encoding
-          rowmax = st->d_rowmax;
-          st->rowmax_valid = true;
-        }
 #define MSB_BUNDLE_ARGS st->d_feats_scalar, (int)st->n_scalar, st->d_params, st->region_rows, (uint32_t)stage_b, Sb, st->d_base_score, \
                         scores, st->ld, org, row_lo, row_hi, st->d_hp, st->d_ss, st->d_col2slot, (int)K, (int)ktiles, rowmax
         if (st->cfg == 1) MSB_BUNDLE_LAUNCH(2, 32, 16);
@@ -1614,7 +1617,6 @@ static int launch_score(msb_state *st, size_t row_lo, size_t row_hi, float *scor
       }
     }
     if (st->cfg == 4) return fail(MSB_ERR_UNSUPPORTED, "score shape 4 exists for the bundled general kernel only");
-    const bool persistent = getenv("MSB_PERSISTENT") != nullptr;   // read per call: the test switches it
     if (blocked && st->tables_only && persistent) {
       // The persistent form of the sweep's tables-only kernel (score_tables_persistent_kernel): one CTA per SM walks
       // (row tile, k-tile) items, the ring runs through the item boundaries, a seventeenth warp is the producer, the
@@ -1646,7 +1648,7 @@ static int launch_score(msb_state *st, size_t row_lo, size_t row_hi, float *scor
     }
     if (smem > ctx->smem_optin) return fail(MSB_ERR_UNSUPPORTED, "score kernel shared memory does not fit");
 #define MSB_SCORE_ARGS st->d_feats_scalar, (int)st->n_scalar, st->d_params, st->region_rows, (uint32_t)stage, S, st->d_base_score, \
-                       scores, st->ld, org, row_lo, row_hi, st->d_hp, st->d_ss, st->d_col2slot, (int)K, (int)ktiles, st->tail_g
+                       scores, st->ld, org, row_lo, row_hi, st->d_hp, st->d_ss, st->d_col2slot, (int)K, (int)ktiles, st->tail_g, rowmax
 #define MSB_SCORE_LAUNCH(V_, RW_, NW_)                                                                         \
     do {                                                                                                       \
       if (blocked && st->tables_only) LAUNCH(ctx, (score_kernel<V_, RW_, NW_, true, true>), (unsigned)grid, NW_ * 32, smem, MSB_SCORE_ARGS);        \
@@ -2175,6 +2177,40 @@ extern "C" MSB_API int msb_state_score_assignment(msb_state *st, float *out) {
 }
 
 // ---- sampler ---------------------------------------------------------------------
+// 32-row tile staged in shared memory (sample_tile_kernel): scores read from HBM exactly once (bulk copy of the
+// blocked layout, or coalesced transposing loads of a row-major one)
+static bool tile_sampler_fits(size_t K) { return K * 33 * 4 <= 48 * 1024 && !getenv("MSB_NO_TILE_SAMPLER"); }
+
+static int launch_tile_sampler(msb_ctx *ctx, bool blocked, const float *scores, size_t ld, size_t skip, int K, size_t nrows,
+                               const float *d_u, uint64_t seed, uint64_t sweep, uint64_t row_id0, const int32_t *col2slot,
+                               int32_t *out_col, int32_t *out_slot, const int *rowmax) {
+  const size_t nblk = (skip + nrows + 31) / 32 - skip / 32;
+  // The kernel is bound by instruction issue and latency, so what counts is warps per SM, and a warp's tile is what
+  // limits them: blocks of four warps waste the remainder (K = 256: 32 KB per warp, one block of four per SM where
+  // seven warps fit), blocks of one warp do not: C4 sample 0.566 -> 0.517 ms.  Four-warp blocks stay where they lose
+  // little -- at equal occupancy they are the faster form (C2: 8 warps in two blocks 0.416 ms, 9 one-warp blocks 0.501).
+  auto warps_per_sm = [&](int sw) {
+    return (size_t)sw * std::min<size_t>(32 / sw, ctx->smem_optin / sample_tile_smem(sw, K, !blocked));
+  };
+  const bool one_warp = 2 * warps_per_sm(1) >= 3 * warps_per_sm(4) && !getenv("MSB_SAMPLER_FOUR_WARPS");
+#define MSB_TILE_SAMPLER(SW)                                                                                                      \
+  do {                                                                                                                        \
+    const size_t smem = sample_tile_smem(SW, K, !blocked);                                                                    \
+    const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(32 / SW, ctx->smem_optin / smem));                           \
+    const unsigned grid = (unsigned)std::min<size_t>((nblk + SW - 1) / SW, (size_t)ctx->sm_count * per_sm);                   \
+    if (blocked)                                                                                                              \
+      LAUNCH(ctx, (sample_tile_kernel<SW, false>), grid, SW * 32, smem, scores, ld, skip, K, nrows, d_u, seed, sweep, row_id0,  \
+             col2slot, out_col, out_slot, rowmax);                                                                            \
+    else                                                                                                                      \
+      LAUNCH(ctx, (sample_tile_kernel<SW, true>), grid, SW * 32, smem, scores, ld, skip, K, nrows, d_u, seed, sweep, row_id0,   \
+             col2slot, out_col, out_slot, (const int *)nullptr);                                                              \
+  } while (0)
+  if (one_warp) MSB_TILE_SAMPLER(1);
+  else MSB_TILE_SAMPLER(4);
+#undef MSB_TILE_SAMPLER
+  return MSB_OK;
+}
+
 extern "C" MSB_API int msb_sample_discrete_log(msb_ctx *ctx, const float *scores, size_t nrows, size_t k, size_t ld,
                                        const float *uniforms, int32_t *out) {
   REQUIRE(ctx && scores && uniforms && out, "NULL argument");
@@ -2188,7 +2224,10 @@ extern "C" MSB_API int msb_sample_discrete_log(msb_ctx *ctx, const float *scores
   CU_TRY(d_o.alloc(nrows));
   CU_TRY(cudaMemcpyAsync(d_s, scores, sizeof(float) * nrows * ld, cudaMemcpyHostToDevice, ctx->stream));
   CU_TRY(cudaMemcpyAsync(d_u, uniforms, sizeof(float) * nrows, cudaMemcpyHostToDevice, ctx->stream));
-  LAUNCH(ctx, sample_kernel, cdiv(nrows, 128), 128, 0, (const float *)d_s, ld, (int)k, nrows, (const float *)d_u, 0ull, 0ull, 0ull, (const int32_t *)nullptr, (int32_t *)d_o, (int32_t *)nullptr);
+  if (tile_sampler_fits(k))
+    MSB_TRY(launch_tile_sampler(ctx, false, d_s, ld, 0, (int)k, nrows, d_u, 0ull, 0ull, 0ull, nullptr, d_o, nullptr, nullptr));
+  else
+    LAUNCH(ctx, sample_kernel, cdiv(nrows, 128), 128, 0, (const float *)d_s, ld, (int)k, nrows, (const float *)d_u, 0ull, 0ull, 0ull, (const int32_t *)nullptr, (int32_t *)d_o, (int32_t *)nullptr);
   CU_TRY(cudaMemcpyAsync(out, d_o, sizeof(int32_t) * nrows, cudaMemcpyDeviceToHost, ctx->stream));
   CU_TRY(cudaStreamSynchronize(ctx->stream));
   return MSB_OK;
@@ -2215,6 +2254,39 @@ extern "C" MSB_API int msb_selftest_expf(msb_ctx *ctx, const float *x, size_t n,
   CU_TRY(cudaMemcpyAsync(d, x, sizeof(float) * n, cudaMemcpyHostToDevice, ctx->stream));
   LAUNCH(ctx, selftest_expf_kernel, cdiv(n, 256), 256, 0, (const float *)d, n, d.p + n);
   CU_TRY(cudaMemcpyAsync(y, d.p + n, sizeof(float) * n, cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(cudaStreamSynchronize(ctx->stream));
+  return MSB_OK;
+}
+
+extern "C" MSB_API int msb_selftest_expf2(msb_ctx *ctx, uint64_t *mismatches) {
+  REQUIRE(ctx && mismatches, "NULL argument");
+  CU_TRY(cudaSetDevice(ctx->device));
+  Scratch<unsigned long long> d;
+  CU_TRY(d.alloc(1));
+  CU_TRY(cudaMemsetAsync(d, 0, sizeof(unsigned long long), ctx->stream));
+  LAUNCH(ctx, selftest_expf2_kernel, cdiv((size_t)EXPF2_LAST_BITS / 2 + 1, 256), 256, 0, (unsigned long long *)d);
+  unsigned long long h = 0;
+  CU_TRY(cudaMemcpyAsync(&h, d, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(cudaStreamSynchronize(ctx->stream));
+  *mismatches = h;
+  return MSB_OK;
+}
+
+extern "C" MSB_API int msb_selftest_skip_rule(msb_ctx *ctx, const uint8_t *e, const float *acc, const float *d, size_t n,
+                                             uint8_t *out) {
+  REQUIRE(ctx && e && acc && d && out, "NULL argument");
+  if (!n) return MSB_OK;
+  CU_TRY(cudaSetDevice(ctx->device));
+  Scratch<float> df;
+  Scratch<uint8_t> db;
+  CU_TRY(df.alloc(2 * n));
+  CU_TRY(db.alloc(2 * n));
+  CU_TRY(cudaMemcpyAsync(df, acc, sizeof(float) * n, cudaMemcpyHostToDevice, ctx->stream));
+  CU_TRY(cudaMemcpyAsync(df.p + n, d, sizeof(float) * n, cudaMemcpyHostToDevice, ctx->stream));
+  CU_TRY(cudaMemcpyAsync(db, e, n, cudaMemcpyHostToDevice, ctx->stream));
+  LAUNCH(ctx, selftest_skip_rule_kernel, cdiv(n, 256), 256, 0, (const uint8_t *)db, (const float *)df, (const float *)(df.p + n), n,
+         db.p + n);
+  CU_TRY(cudaMemcpyAsync(out, db.p + n, n, cudaMemcpyDeviceToHost, ctx->stream));
   CU_TRY(cudaStreamSynchronize(ctx->stream));
   return MSB_OK;
 }
@@ -2404,38 +2476,11 @@ extern "C" MSB_API int msb_state_sweep(msb_state *st, size_t row_lo, size_t row_
       CU_TRY(cudaMemcpyAsync(st->d_uniforms, opts->uniforms + (lo - row_lo), sizeof(float) * (hi - lo), cudaMemcpyHostToDevice, ctx->stream));
       d_u = st->d_uniforms;
     }
-    const bool tile_fits = K * 33 * 4 <= 48 * 1024 && !getenv("MSB_NO_TILE_SAMPLER");
-    if (tile_fits) {
-      // 32-row tile staged in shared memory: scores read from HBM exactly once (bulk copy of the blocked layout,
-      // or coalesced transposing loads of the row-major one the NIW kernels write)
-      const size_t tile_bytes = (K * (blocked ? 32 : 33) * 4 + 127) / 128 * 128;
-      const size_t skip_t = blocked ? skip : 0;  // the row-major pointer below already starts at the first valid row
-      const size_t nblk = (skip_t + (hi - lo) + 31) / 32 - skip_t / 32;
-      // The kernel is bound by instruction issue and latency, so what counts is warps per SM, and a warp's tile is what
-      // limits them: blocks of four warps waste the remainder (K = 256: 32 KB per warp, one block of four per SM where
-      // seven warps fit), blocks of one warp do not: C4 sample 0.566 -> 0.517 ms.  Four-warp blocks stay where they lose
-      // little -- at equal occupancy they are the faster form (C2: 8 warps in two blocks 0.416 ms, 9 one-warp blocks 0.501).
-      auto warps_per_sm = [&](int sw) {
-        const size_t smem = (size_t)sw * tile_bytes + sw * sizeof(uint64_t) + 64;
-        return (size_t)sw * std::min<size_t>(32 / sw, ctx->smem_optin / smem);
-      };
-      const bool one_warp = 2 * warps_per_sm(1) >= 3 * warps_per_sm(4) && !getenv("MSB_SAMPLER_FOUR_WARPS");
-#define MSB_TILE_SAMPLER(SW)                                                                                                      \
-      do {                                                                                                                        \
-        const size_t smem = (size_t)SW * tile_bytes + SW * sizeof(uint64_t) + 64;                                                 \
-        const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(32 / SW, ctx->smem_optin / smem));                           \
-        const unsigned grid = (unsigned)std::min<size_t>((nblk + SW - 1) / SW, (size_t)ctx->sm_count * per_sm);                   \
-        if (blocked)                                                                                                              \
-          LAUNCH(ctx, (sample_tile_kernel<SW, false>), grid, SW * 32, smem, st->d_scores, st->ld, skip, (int)K, hi - lo, d_u, opts->seed, \
-                 opts->sweep, opts->row_id_offset + lo, st->d_col2slot, st->d_newcol, st->d_newslot);                             \
-        else                                                                                                                      \
-          LAUNCH(ctx, (sample_tile_kernel<SW, true>), grid, SW * 32, smem, st->d_scores + skip * st->ld, st->ld, (size_t)0, (int)K, hi - lo, \
-                 d_u, opts->seed, opts->sweep, opts->row_id_offset + lo, st->d_col2slot, st->d_newcol, st->d_newslot);            \
-      } while (0)
-      if (one_warp) MSB_TILE_SAMPLER(1);
-      else MSB_TILE_SAMPLER(4);
-#undef MSB_TILE_SAMPLER
-    } else if (blocked)
+    if (tile_sampler_fits(K))
+      MSB_TRY(launch_tile_sampler(ctx, blocked, st->d_scores + (blocked ? 0 : skip * st->ld), st->ld, blocked ? skip : 0, (int)K,
+                                  hi - lo, d_u, opts->seed, opts->sweep, opts->row_id_offset + lo, st->d_col2slot, st->d_newcol,
+                                  st->d_newslot, blocked && st->rowmax_valid ? st->d_rowmax : nullptr));
+    else if (blocked)
       LAUNCH(ctx, sample_blocked_kernel, cdiv(hi - lo, 128), 128, 0, st->d_scores, st->ld, skip, (int)K, hi - lo, d_u, opts->seed,
              opts->sweep, opts->row_id_offset + lo, st->d_col2slot, st->d_newcol, st->d_newslot,
              (const int *)(st->rowmax_valid ? st->d_rowmax : nullptr));

@@ -231,8 +231,15 @@ MSB_API int msb_philox_uniforms(msb_ctx *ctx, uint64_t seed, uint64_t sweep, uin
 /* y[i] = the sampler's exp (DESIGN.md, sampler contract) of x[i], evaluated on the device: the checker's own copy
  * must give the same bits */
 MSB_API int msb_selftest_expf(msb_ctx *ctx, const float *x, size_t n, float *y);
-/* device self-test of the sampler's division sequence (DESIGN.md, sampler contract): n pseudo-random operand
- * pairs, counts the results that differ from the IEEE division.  Must report 0. */
+/* device self-test of the sampler's packed exp (DESIGN.md, sampler contract): every float x in [-86, 0] through the
+ * two-at-a-time form and through the scalar one; counts the results whose bits differ.  Must report 0. */
+MSB_API int msb_selftest_expf2(msb_ctx *ctx, uint64_t *mismatches);
+/* out[i] = 1 where the sampler's dart walk would skip a batch whose largest p has the biased exponent e[i], for a sum
+ * acc[i] and a dart d[i] (DESIGN.md, sampler contract), else 0; evaluated on the device so that the host can check the
+ * rule exactly */
+MSB_API int msb_selftest_skip_rule(msb_ctx *ctx, const uint8_t *e, const float *acc, const float *d, size_t n, uint8_t *out);
+/* device self-test of the sampler's division sequence (DESIGN.md, sampler contract), scalar and packed: n pseudo-random
+ * operand sets, counts the results that differ from the IEEE division.  Must report 0. */
 MSB_API int msb_selftest_division(msb_ctx *ctx, uint64_t seed, size_t n, uint64_t *mismatches);
 
 typedef struct msb_sweep_opts {
