@@ -56,6 +56,15 @@ class SweepResult(C.Structure):
     _fields_ = [("rows", C.c_uint64), ("moved", C.c_uint64), ("units", C.c_uint64)]
 
 
+class PredictOpts(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("counter", C.c_uint64), ("row_id_offset", C.c_uint64), ("uniforms", C.c_void_p)]
+
+
+class PredictOut(C.Structure):
+    _fields_ = [("logp", C.c_void_p), ("resp", C.c_void_p), ("resp_ld", C.c_size_t), ("map_gid", C.c_void_p),
+                ("draw_gid", C.c_void_p), ("values", C.c_void_p), ("values_ld", C.c_size_t)]
+
+
 _P = C.c_void_p
 _SZ = C.c_size_t
 _PROTOS = {
@@ -119,6 +128,8 @@ _PROTOS = {
     "msb_selftest_skip_rule": (C.c_int, [_P, _P, _P, _P, _SZ, _P]),
     "msb_state_sweep": (C.c_int, [_P, _SZ, _SZ, C.POINTER(SweepOpts), C.POINTER(SweepResult)]),
     "msb_state_sweep_wait": (C.c_int, [_P, C.POINTER(SweepResult)]),
+    "msb_state_predict": (C.c_int, [_P, _SZ, _SZ, C.POINTER(PredictOpts), C.POINTER(PredictOut), C.POINTER(_SZ), _SZ,
+                                    C.POINTER(_SZ)]),
     "msb_state_delta_buffer": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),
     "msb_state_apply_deltas": (C.c_int, [_P]),
     "msb_state_delta_buffer_i32": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),

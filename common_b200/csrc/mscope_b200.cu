@@ -22,6 +22,7 @@
 #include "msb_niw_tc.cuh"
 #include "msb_niw_tc16.cuh"
 #include "msb_draw.cuh"
+#include "msb_predict.cuh"
 
 using namespace msb;
 
@@ -279,6 +280,10 @@ extern "C" MSB_API int msb_ctx_create(int device, void *stream, msb_ctx **out) {
   CU_TRY(opt_in_smem((sample_tile_kernel<4, true>), c->smem_optin));
   CU_TRY(opt_in_smem((sample_tile_kernel<1, false>), c->smem_optin));
   CU_TRY(opt_in_smem((sample_tile_kernel<1, true>), c->smem_optin));
+  CU_TRY(opt_in_smem((predict_tile_kernel<4, false>), c->smem_optin));
+  CU_TRY(opt_in_smem((predict_tile_kernel<4, true>), c->smem_optin));
+  CU_TRY(opt_in_smem((predict_tile_kernel<1, false>), c->smem_optin));
+  CU_TRY(opt_in_smem((predict_tile_kernel<1, true>), c->smem_optin));
   CU_TRY(opt_in_smem((ingest_tile_kernel<512, 1>), c->smem_optin));
   CU_TRY(opt_in_smem((ingest_tile_kernel<256, 2>), c->smem_optin));
   CU_TRY(opt_in_smem((ingest_tile_kernel<128, 4>), c->smem_optin));
@@ -2425,6 +2430,50 @@ extern "C" MSB_API int msb_state_last_allreduce_bytes(msb_state *st, size_t *byt
 }
 
 // ---- sweep -------------------------------------------------------------------------
+// rows per chunk of a sweep or a prediction: the score matrix of one chunk stays within MSB_SCORES_MB (default 4 GB)
+static size_t score_chunk_rows(const msb_state *st, size_t nrows) {
+  size_t budget_mb = 4096;
+  if (const char *e = getenv("MSB_SCORES_MB")) budget_mb = std::max(1, atoi(e));
+  size_t chunk = std::max<size_t>(1, std::min(nrows, budget_mb * 1024 * 1024 / (st->ld * sizeof(float))));
+  if (chunk < nrows) chunk = std::max<size_t>(1024, chunk / 1024 * 1024);
+  return chunk;
+}
+
+// the sweep keeps the scores in the sampler-friendly blocked layout; the CUDA-core NIW kernel (dim != 64)
+// accumulates row-major only
+static bool blocked_layout(const msb_state *st) {
+  bool niw_tc_only = true;
+  for (const auto &f : st->feats) if (f.kind == KIND_NIW && (f.dim != 64 || getenv("MSB_NO_TENSOR"))) niw_tc_only = false;
+  if (st->has_dm) niw_tc_only = false;  // dm_score_kernel accumulates row-major
+  return niw_tc_only && !getenv("MSB_NO_BLOCKED");
+}
+
+// one group per row of the chunk [lo, hi) of a call over [row_lo, row_hi), from the score matrix launch_score left in
+// d_scores: column into d_newcol, slot into d_newslot.  uniforms (host, one per row of the call) or NULL -> Philox
+// (seed, row_id_offset + row, counter).
+static int launch_sampler(msb_state *st, bool blocked, size_t K, size_t row_lo, size_t lo, size_t hi, const float *uniforms,
+                          uint64_t seed, uint64_t counter, uint64_t row_id_offset) {
+  msb_ctx *ctx = st->ctx;
+  const size_t skip = lo - row_origin(lo);
+  const float *d_u = nullptr;
+  if (uniforms) {
+    CU_TRY(cudaMemcpyAsync(st->d_uniforms, uniforms + (lo - row_lo), sizeof(float) * (hi - lo), cudaMemcpyHostToDevice, ctx->stream));
+    d_u = st->d_uniforms;
+  }
+  if (tile_sampler_fits(K))
+    MSB_TRY(launch_tile_sampler(ctx, blocked, st->d_scores + (blocked ? 0 : skip * st->ld), st->ld, blocked ? skip : 0, (int)K,
+                                hi - lo, d_u, seed, counter, row_id_offset + lo, st->d_col2slot, st->d_newcol,
+                                st->d_newslot, blocked && st->rowmax_valid ? st->d_rowmax : nullptr));
+  else if (blocked)
+    LAUNCH(ctx, sample_blocked_kernel, cdiv(hi - lo, 128), 128, 0, st->d_scores, st->ld, skip, (int)K, hi - lo, d_u, seed,
+           counter, row_id_offset + lo, st->d_col2slot, st->d_newcol, st->d_newslot,
+           (const int *)(st->rowmax_valid ? st->d_rowmax : nullptr));
+  else
+    LAUNCH(ctx, sample_kernel, cdiv(hi - lo, 128), 128, 0, st->d_scores + skip * st->ld, st->ld, (int)K, hi - lo, d_u, seed,
+           counter, row_id_offset + lo, st->d_col2slot, st->d_newcol, st->d_newslot);
+  return MSB_OK;
+}
+
 extern "C" MSB_API int msb_state_sweep(msb_state *st, size_t row_lo, size_t row_hi, const msb_sweep_opts *opts,
                                msb_sweep_result *res) {
   REQUIRE(st && opts, "NULL argument");
@@ -2437,10 +2486,7 @@ extern "C" MSB_API int msb_state_sweep(msb_state *st, size_t row_lo, size_t row_
   const size_t nrows = row_hi - row_lo;
   if (res) { res->rows = nrows; res->moved = 0; res->units = (uint64_t)nrows * K * st->D; }
   if (!nrows) return MSB_OK;
-  size_t budget_mb = 4096;
-  if (const char *e = getenv("MSB_SCORES_MB")) budget_mb = std::max(1, atoi(e));
-  size_t chunk = std::max<size_t>(1, std::min(nrows, budget_mb * 1024 * 1024 / (st->ld * sizeof(float))));
-  if (chunk < nrows) chunk = std::max<size_t>(1024, chunk / 1024 * 1024);
+  const size_t chunk = score_chunk_rows(st, nrows);
   const size_t nchunks = (nrows + chunk - 1) / chunk;
   MSB_TRY(ensure_scores(st, chunk + 128));
   MSB_TRY(ensure_rows(st, chunk));
@@ -2453,12 +2499,7 @@ extern "C" MSB_API int msb_state_sweep(msb_state *st, size_t row_lo, size_t row_
   }
   st->ring_nchunks[ring] = nchunks;
   st->sweep_seq++;
-  // the sweep keeps the scores in the sampler-friendly blocked layout; the CUDA-core NIW kernel (dim != 64)
-  // accumulates row-major only
-  bool niw_tc_only = true;
-  for (const auto &f : st->feats) if (f.kind == KIND_NIW && (f.dim != 64 || getenv("MSB_NO_TENSOR"))) niw_tc_only = false;
-  if (st->has_dm) niw_tc_only = false;  // dm_score_kernel accumulates row-major
-  const bool blocked = niw_tc_only && !getenv("MSB_NO_BLOCKED");
+  const bool blocked = blocked_layout(st);
   LAUNCH(ctx, zero_u64_kernel, 1, 1, 0, st->d_counter);
   CU_TRY(cudaEventRecord(ev[0].e[0], ctx->stream));
   MSB_TRY(build_params(st));
@@ -2471,22 +2512,7 @@ extern "C" MSB_API int msb_state_sweep(msb_state *st, size_t row_lo, size_t row_
     MSB_TRY(launch_score(st, lo, hi, st->d_scores, blocked, true));
     st->last_skip = skip;
     CU_TRY(cudaEventRecord(pe.e[1], ctx->stream));
-    const float *d_u = nullptr;
-    if (opts->uniforms) {
-      CU_TRY(cudaMemcpyAsync(st->d_uniforms, opts->uniforms + (lo - row_lo), sizeof(float) * (hi - lo), cudaMemcpyHostToDevice, ctx->stream));
-      d_u = st->d_uniforms;
-    }
-    if (tile_sampler_fits(K))
-      MSB_TRY(launch_tile_sampler(ctx, blocked, st->d_scores + (blocked ? 0 : skip * st->ld), st->ld, blocked ? skip : 0, (int)K,
-                                  hi - lo, d_u, opts->seed, opts->sweep, opts->row_id_offset + lo, st->d_col2slot, st->d_newcol,
-                                  st->d_newslot, blocked && st->rowmax_valid ? st->d_rowmax : nullptr));
-    else if (blocked)
-      LAUNCH(ctx, sample_blocked_kernel, cdiv(hi - lo, 128), 128, 0, st->d_scores, st->ld, skip, (int)K, hi - lo, d_u, opts->seed,
-             opts->sweep, opts->row_id_offset + lo, st->d_col2slot, st->d_newcol, st->d_newslot,
-             (const int *)(st->rowmax_valid ? st->d_rowmax : nullptr));
-    else
-      LAUNCH(ctx, sample_kernel, cdiv(hi - lo, 128), 128, 0, st->d_scores + skip * st->ld, st->ld, (int)K, hi - lo, d_u, opts->seed,
-             opts->sweep, opts->row_id_offset + lo, st->d_col2slot, st->d_newcol, st->d_newslot);
+    MSB_TRY(launch_sampler(st, blocked, K, row_lo, lo, hi, opts->uniforms, opts->seed, opts->sweep, opts->row_id_offset));
     CU_TRY(cudaEventRecord(pe.e[2], ctx->stream));
     MSB_TRY(launch_update(st, lo, hi));
     CU_TRY(cudaEventRecord(pe.e[3], ctx->stream));
@@ -2515,6 +2541,139 @@ extern "C" MSB_API int msb_state_sweep_wait(msb_state *st, msb_sweep_result *res
   CU_TRY(cudaStreamSynchronize(st->ctx->stream));
   st->last_res.moved = *st->h_moved;
   if (res) *res = st->last_res;
+  return MSB_OK;
+}
+
+// ---- posterior predictive of a row range (DESIGN.md section 4.9) ------------------------------------------------------
+// logp / resp / MAP from one score matrix: the 32-row tile form where a tile fits (as the sampler), else one thread per row
+static int launch_predict(msb_state *st, bool blocked, int K, size_t lo, size_t hi, const double *d_logz, double *logp,
+                          int32_t *map_col, float *resp) {
+  msb_ctx *ctx = st->ctx;
+  const size_t nrows = hi - lo, skip = lo - row_origin(lo);
+  const float *scores = st->d_scores + (blocked ? 0 : skip * st->ld);
+  const size_t sk = blocked ? skip : 0;
+  const int *rowmax = blocked && st->rowmax_valid ? st->d_rowmax : nullptr;
+  if (!tile_sampler_fits(K)) {
+    if (blocked)
+      LAUNCH(ctx, predict_rows_kernel<false>, cdiv(nrows, 128), 128, 0, scores, st->ld, sk, K, nrows, rowmax, d_logz, logp, map_col, resp, (size_t)K);
+    else
+      LAUNCH(ctx, predict_rows_kernel<true>, cdiv(nrows, 128), 128, 0, scores, st->ld, sk, K, nrows, rowmax, d_logz, logp, map_col, resp, (size_t)K);
+    return MSB_OK;
+  }
+  const size_t nblk = (sk + nrows + 31) / 32 - sk / 32;
+  // warps per SM, as launch_tile_sampler chooses them: one-warp blocks where four-warp blocks would waste shared memory
+  auto warps_per_sm = [&](int sw) { return (size_t)sw * std::min<size_t>(32 / sw, ctx->smem_optin / predict_tile_smem(sw, K, !blocked)); };
+  const bool one_warp = 2 * warps_per_sm(1) >= 3 * warps_per_sm(4);
+#define MSB_PREDICT_TILE(SW)                                                                                                  \
+  do {                                                                                                                    \
+    const size_t smem = predict_tile_smem(SW, K, !blocked);                                                               \
+    const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(32 / SW, ctx->smem_optin / smem));                       \
+    const unsigned grid = (unsigned)std::min<size_t>((nblk + SW - 1) / SW, (size_t)ctx->sm_count * per_sm);               \
+    if (blocked)                                                                                                          \
+      LAUNCH(ctx, (predict_tile_kernel<SW, false>), grid, SW * 32, smem, scores, st->ld, sk, K, nrows, rowmax, d_logz, logp, map_col, resp, (size_t)K); \
+    else                                                                                                                  \
+      LAUNCH(ctx, (predict_tile_kernel<SW, true>), grid, SW * 32, smem, scores, st->ld, sk, K, nrows, (const int *)nullptr, d_logz, logp, map_col, resp, (size_t)K); \
+  } while (0)
+  if (one_warp) MSB_PREDICT_TILE(1);
+  else MSB_PREDICT_TILE(4);
+#undef MSB_PREDICT_TILE
+  return MSB_OK;
+}
+
+extern "C" MSB_API int msb_state_predict(msb_state *st, size_t row_lo, size_t row_hi, const msb_predict_opts *opts,
+                                         msb_predict_out *out, size_t *gids, size_t cap, size_t *ncols) {
+  REQUIRE(st && opts && out && ncols, "NULL argument");
+  REQUIRE(st->dv, "no dataview bound");
+  REQUIRE(row_lo <= row_hi && row_hi <= st->n, "bad row range");
+  msb_ctx *ctx = st->ctx;
+  CU_TRY(cudaSetDevice(ctx->device));
+  MSB_TRY(prepare_columns(st));
+  const size_t K = st->h_col2slot.size(), D = st->D;
+  *ncols = K;
+  if (gids) { REQUIRE(cap >= K, "buffer too small"); for (size_t c = 0; c < K; c++) gids[c] = st->h_colgid[c]; }
+  REQUIRE(!out->resp || out->resp_ld >= K, "resp_ld smaller than the number of groups");
+  std::vector<ImputeFeat> ifeat(D);
+  size_t W = 0;
+  for (size_t d = 0; d < D; d++) {
+    ifeat[d].off = W; ifeat[d].fac = nullptr;
+    W += (st->feats[d].kind == KIND_NIW || st->feats[d].kind == KIND_DM) ? st->feats[d].dim : 1;
+  }
+  const bool impute = out->values != nullptr;
+  const bool draw = impute || out->draw_gid;
+  if (impute) {
+    REQUIRE(out->values_ld >= W, "values_ld smaller than the row width");
+    // the draw counters counter * 2^40 + row id * D + d must not overlap between counters
+    REQUIRE(opts->counter < (1ull << 24), "counter must be below 2^24 for imputation");
+    REQUIRE(opts->row_id_offset + row_hi <= ((1ull << 40) - 1) / std::max<size_t>(D, 1), "row ids times features must stay below 2^40");
+  }
+  const size_t nrows = row_hi - row_lo;
+  if (!nrows) return MSB_OK;
+  const size_t chunk = score_chunk_rows(st, nrows);
+  const size_t nchunks = (nrows + chunk - 1) / chunk;
+  MSB_TRY(ensure_scores(st, chunk + 128));
+  MSB_TRY(ensure_rows(st, chunk));
+  const bool blocked = blocked_layout(st);
+  MSB_TRY(build_params(st));
+  Scratch<double> d_logz, d_logp, d_vals;
+  Scratch<int32_t> d_map;
+  Scratch<float> d_resp;
+  Scratch<uint32_t> d_unsupported;
+  Scratch<ImputeFeat> d_ifeat;
+  std::vector<Scratch<double>> d_fac(D);
+  CU_TRY(d_logz.alloc(1));
+  CU_TRY(d_logp.alloc(chunk));
+  CU_TRY(d_map.alloc(chunk));
+  if (out->resp) CU_TRY(d_resp.alloc(chunk * K));
+  LAUNCH(ctx, crp_logz_kernel, 1, 256, 0, st->d_ss, st->d_col2slot, (int)K, (float)st->alpha, d_logz.p);
+  if (impute) {
+    CU_TRY(d_vals.alloc(chunk * W));
+    CU_TRY(d_unsupported.alloc(1));
+    CU_TRY(cudaMemsetAsync(d_unsupported, 0, sizeof(uint32_t), ctx->stream));
+    for (size_t d = 0; d < D; d++) {
+      const FeatDev &f = st->feats[d];
+      if (f.kind != KIND_NIW) continue;
+      const size_t smem = ((size_t)f.dim * f.dim + f.dim) * sizeof(double);
+      if (smem > 48 * 1024) CU_TRY(cudaFuncSetAttribute(niw_predictive_factor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      CU_TRY(d_fac[d].alloc(st->kmax * ((size_t)f.dim * f.dim + f.dim + 1)));
+      LAUNCH(ctx, niw_predictive_factor_kernel, (unsigned)K, 128, smem, f, st->d_hp, st->d_ss, st->d_col2slot, d_fac[d].p);
+      ifeat[d].fac = d_fac[d].p;
+    }
+    CU_TRY(d_ifeat.alloc(D));
+    CU_TRY(cudaMemcpyAsync(d_ifeat.p, ifeat.data(), sizeof(ImputeFeat) * D, cudaMemcpyHostToDevice, ctx->stream));
+  }
+  std::vector<int32_t> h_map(chunk), h_draw(draw ? chunk : 0);
+  for (size_t c = 0; c < nchunks; c++) {
+    const size_t lo = row_lo + c * chunk, hi = std::min(row_hi, lo + chunk), n = hi - lo, r0 = lo - row_lo;
+    MSB_TRY(launch_score(st, lo, hi, st->d_scores, blocked, true));
+    MSB_TRY(launch_predict(st, blocked, (int)K, lo, hi, d_logz, d_logp, d_map, d_resp));
+    if (draw) MSB_TRY(launch_sampler(st, blocked, K, row_lo, lo, hi, opts->uniforms, opts->seed, opts->counter, opts->row_id_offset));
+    if (impute)
+      LAUNCH(ctx, impute_kernel, dim3(cdiv(n, 128), (unsigned)D), 128, 0, st->d_feats, (const ImputeFeat *)d_ifeat.p, (int)D,
+             st->d_hp, st->d_ss, st->d_newslot, lo, n, opts->seed, opts->counter << 40, opts->row_id_offset + lo, d_vals.p, W,
+             d_unsupported.p);
+    if (out->logp) CU_TRY(cudaMemcpyAsync(out->logp + r0, d_logp, sizeof(double) * n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (out->map_gid) CU_TRY(cudaMemcpyAsync(h_map.data(), d_map, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (draw) CU_TRY(cudaMemcpyAsync(h_draw.data(), st->d_newcol, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (out->resp)
+      CU_TRY(cudaMemcpy2DAsync(out->resp + r0 * out->resp_ld, sizeof(float) * out->resp_ld, d_resp, sizeof(float) * K, sizeof(float) * K,
+                               n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (impute)
+      CU_TRY(cudaMemcpy2DAsync(out->values + r0 * out->values_ld, sizeof(double) * out->values_ld, d_vals, sizeof(double) * W,
+                               sizeof(double) * W, n, cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(cudaStreamSynchronize(ctx->stream));
+    for (size_t i = 0; i < n; i++) {
+      if (out->map_gid) out->map_gid[r0 + i] = (int64_t)st->h_colgid[h_map[i]];
+      if (out->draw_gid) out->draw_gid[r0 + i] = (int64_t)st->h_colgid[h_draw[i]];
+    }
+    st->last_skip = lo - row_origin(lo);
+  }
+  st->last_rows = nchunks == 1 ? nrows : (nrows - (nchunks - 1) * chunk); st->last_cols = K;
+  st->last_blocked = blocked;
+  if (impute) {
+    uint32_t bad = 0;
+    CU_TRY(cudaMemcpy(&bad, d_unsupported, sizeof(bad), cudaMemcpyDeviceToHost));
+    if (bad) return fail(MSB_ERR_UNSUPPORTED, "multinomial sampling unimplemented");  // dm.cpp:100-111
+  }
   return MSB_OK;
 }
 

@@ -252,6 +252,50 @@ class state(object):
         _lib.check(_lib.load().msb_state_sweep_wait(self._h, C.byref(res)))
         return {"rows": res.rows, "moved": res.moved, "units": res.units}
 
+    def predict(self, row_lo=0, row_hi=None, *, responsibilities=False, map=False, draw=False, impute=False, seed=0,
+                counter=0, row_id_offset=0, uniforms=None):
+        """posterior predictive of rows [row_lo, row_hi) of the bound dataview against the current suffstats (an assigned
+        row's own contribution included: not leave-one-out).  Returns a dict with ``gids`` (the columns), ``logp``
+        (log p(x_observed | state), float64), and where asked ``resp`` (float32 [nrows, K], the sampler's own
+        probabilities), ``map_gid``, ``draw_gid`` (the sweep's draw with sweep word ``counter``) and ``values`` (one array
+        per feature, [nrows] or [nrows, dim]: observed cells as stored, masked cells drawn from the drawn group's
+        posterior predictive).  Nothing of the state changes."""
+        row_hi = self.nentities() if row_hi is None else row_hi
+        n = row_hi - row_lo
+        k = self.ngroups()
+        widths = [m._param() if m.name() in ("niw", "dm") else 1 for m in self._models]
+        res = {"logp": np.zeros(n, np.float64)}
+        out = _lib.PredictOut()
+        out.logp = res["logp"].ctypes.data
+        if responsibilities:
+            res["resp"] = np.zeros((n, k), np.float32)
+            out.resp, out.resp_ld = res["resp"].ctypes.data, k
+        if map:
+            res["map_gid"] = np.zeros(n, np.int64)
+            out.map_gid = res["map_gid"].ctypes.data
+        if draw or impute:
+            res["draw_gid"] = np.zeros(n, np.int64)
+            out.draw_gid = res["draw_gid"].ctypes.data
+        if impute:
+            vals = np.zeros((n, sum(widths)), np.float64)
+            out.values, out.values_ld = vals.ctypes.data, vals.shape[1]
+        opts = _lib.PredictOpts(int(seed), int(counter), int(row_id_offset), None)
+        keep = None
+        if uniforms is not None:
+            keep = np.ascontiguousarray(uniforms, dtype=np.float32)
+            assert keep.size == n
+            opts.uniforms = keep.ctypes.data
+        gids = (C.c_size_t * max(k, 1))()
+        nc = C.c_size_t()
+        _lib.check(_lib.load().msb_state_predict(self._h, row_lo, row_hi, C.byref(opts), C.byref(out), gids, k, C.byref(nc)))
+        res["gids"] = [int(gids[i]) for i in range(nc.value)]
+        if impute:
+            res["values"], off = [], 0
+            for m, w in zip(self._models, widths):
+                res["values"].append(vals[:, off:off + w] if m.name() in ("niw", "dm") else vals[:, off])
+                off += w
+        return res
+
     def last_scores(self):
         """(device pointer, ld, nrows, ncols) of the score matrix the last score/sweep call wrote"""
         ptr, ld, nr, nc = C.c_void_p(), C.c_size_t(), C.c_size_t(), C.c_size_t()

@@ -285,6 +285,34 @@ public:
     if (gids) *gids = g;
     return out;
   }
+  // posterior predictive of rows [row_lo, row_hi) (msb_state_predict): logp always; resp ([nrows][K]), map / draw gids and
+  // the imputed values ([nrows][W], masked cells drawn from the drawn group) when the pointer is non-null
+  std::vector<double> predict(size_t row_lo, size_t row_hi, uint64_t seed = 0, uint64_t counter = 0,
+                              std::vector<float> *resp = nullptr, std::vector<int64_t> *map_gid = nullptr,
+                              std::vector<int64_t> *draw_gid = nullptr, std::vector<double> *values = nullptr,
+                              std::vector<size_t> *gids = nullptr) {
+    size_t k = 0;
+    b200::check(msb_state_ngroups(st_, &k));
+    size_t w = 0;
+    for (const auto &m : descs_) w += (m.family == MSB_FAMILY_NIW || m.family == MSB_FAMILY_DM) ? m.dim : 1;
+    const size_t n = row_hi - row_lo;
+    std::vector<double> logp(n);
+    msb_predict_opts o;
+    std::memset(&o, 0, sizeof(o));
+    o.seed = seed; o.counter = counter;
+    msb_predict_out out;
+    std::memset(&out, 0, sizeof(out));
+    out.logp = logp.data();
+    if (resp) { resp->assign(n * k, 0.f); out.resp = resp->data(); out.resp_ld = k; }
+    if (map_gid) { map_gid->assign(n, -1); out.map_gid = map_gid->data(); }
+    if (draw_gid) { draw_gid->assign(n, -1); out.draw_gid = draw_gid->data(); }
+    if (values) { values->assign(n * w, 0.0); out.values = values->data(); out.values_ld = w; }
+    std::vector<size_t> g(k);
+    size_t ncols = 0;
+    b200::check(msb_state_predict(st_, row_lo, row_hi, &o, &out, g.data(), k, &ncols));
+    if (gids) *gids = g;
+    return logp;
+  }
   msb_sweep_result sweep(uint64_t seed, uint64_t sweep_id) {
     msb_sweep_opts o;
     std::memset(&o, 0, sizeof(o));

@@ -27,6 +27,8 @@
  *                         common/util.hpp:125-156 (scores_to_probs + sample_discrete)
  *   msb_state_sweep       one batched (synchronous, approximate) reassignment pass: score/sample/update
  *                         (SURVEY.md section 3b) against frozen suffstats
+ *   msb_state_predict     mixturemodel's score_value (logsumexp of one inplace_score_value over the groups), the
+ *                         responsibilities, and sample_post_pred's imputation of masked cells, for a row range
  *   msb_value_*           single-value group::score_value/add_value/remove_value/score_data/sample_value
  *                         (models/base.hpp:25-27), executed on the device
  *
@@ -274,6 +276,43 @@ MSB_API int msb_state_sweep(msb_state *st, size_t row_lo, size_t row_hi, const m
 
 /* waits for the stream and reports the last sweep (rows, moved, units) */
 MSB_API int msb_state_sweep_wait(msb_state *st, msb_sweep_result *res);
+
+/* ---- posterior predictive of rows [row_lo, row_hi) of the bound dataview (DESIGN.md section 4.9) ---------------------
+ * The rows are scored against the current suffstats exactly as msb_state_score_rows scores them (columns c <-> gids[c],
+ * ascending gid).  An assigned row's own contribution is part of the suffstats it is scored against: this is not a
+ * leave-one-out predictive.  Held-out rows are bound unassigned (add_values with -1) and swept around.
+ * For a row with fp32 scores s_c: m = max s_c, p_c = the sampler's exp(s_c - m), acc = sum p_c in fp64, column order.
+ *   logp      log p(x_observed | state) = m + log(acc) - log(Z), Z = sum of the pseudocounts (fp64): with an empty group
+ *             Z = N_assigned + alpha and logp is the DP posterior predictive (the existing clusters and a new one); with
+ *             none it is the finite mixture over the present groups.  Replaces score_rows + the CRP normaliser + a host
+ *             logsumexp (mixturemodel's score_value).
+ *   resp      RN(p_c / (float)acc): bit for bit the probabilities the sampler walks (util.hpp:125-136).  Replaces
+ *             score_rows + scores_to_probs on the host.
+ *   map_gid   the gid of the first column with s_c = m.
+ *   draw_gid  the sweep's draw for the row, uniform philox_u01(seed, row_id_offset + row, counter) or uniforms[row - row_lo].
+ *             Replaces score_rows + msb_sample_discrete_log.
+ *   values    [nrows][values_ld >= W], W = sum of the feature widths (dim for niw and dm, else 1), feature order: an
+ *             observed cell is the value the device holds (the cast column value); a masked one (as the scorer sees it:
+ *             a dd category outside [0, C), a niw vector with any masked element) is drawn from the posterior predictive
+ *             of the row's drawn group, equal to msb_state_sample_value(d, gid, seed, counter * 2^40 + (row_id_offset +
+ *             row) * D + d, n = 1).  Implies the draw.  counter >= 2^24 or (row_id_offset + row_hi) * D >= 2^40:
+ *             MSB_ERR_INVALID.  A masked dm cell: MSB_ERR_UNSUPPORTED, "multinomial sampling unimplemented".  Replaces
+ *             one msb_state_sample_value call per masked cell (sample_post_pred).
+ * Every output is optional (NULL: not wanted).  Nothing of the state changes: assignments, suffstats, deltas, counts
+ * and the sweep timing ring stay as they are; msb_state_last_scores describes the matrix of the last row chunk scored. */
+typedef struct msb_predict_opts {
+  uint64_t seed, counter, row_id_offset;
+  const float *uniforms;              /* host, one per row of [row_lo, row_hi), or NULL -> Philox */
+} msb_predict_opts;
+typedef struct msb_predict_out {      /* host pointers; NULL = not wanted */
+  double *logp;                       /* [nrows] */
+  float *resp; size_t resp_ld;        /* [nrows][resp_ld >= K], column c <-> gids[c] */
+  int64_t *map_gid;                   /* [nrows] */
+  int64_t *draw_gid;                  /* [nrows] */
+  double *values; size_t values_ld;   /* [nrows][values_ld >= W] */
+} msb_predict_out;
+MSB_API int msb_state_predict(msb_state *st, size_t row_lo, size_t row_hi, const msb_predict_opts *opts,
+                              msb_predict_out *out, size_t *gids, size_t cap, size_t *ncols);
 
 /* multi-GPU: flat fp64 buffer [group counts | per-feature suffstat deltas] on the device */
 MSB_API int msb_state_delta_buffer(msb_state *st, double **dev_ptr, size_t *count);
