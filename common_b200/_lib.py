@@ -65,6 +65,14 @@ class PredictOut(C.Structure):
                 ("draw_gid", C.c_void_p), ("values", C.c_void_p), ("values_ld", C.c_size_t)]
 
 
+class HpGibbsOpts(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("counter", C.c_uint64)]
+
+
+class HpGibbsOut(C.Structure):
+    _fields_ = [("choice", C.c_void_p), ("logw", C.c_void_p), ("logw_ld", C.c_size_t)]
+
+
 _P = C.c_void_p
 _SZ = C.c_size_t
 _PROTOS = {
@@ -130,6 +138,9 @@ _PROTOS = {
     "msb_state_sweep_wait": (C.c_int, [_P, C.POINTER(SweepResult)]),
     "msb_state_predict": (C.c_int, [_P, _SZ, _SZ, C.POINTER(PredictOpts), C.POINTER(PredictOut), C.POINTER(_SZ), _SZ,
                                     C.POINTER(_SZ)]),
+    "msb_state_set_hp_grid": (C.c_int, [_P, _SZ, C.POINTER(C.c_double), _SZ, _SZ, C.POINTER(C.c_double)]),
+    "msb_state_set_cluster_hp_grid": (C.c_int, [_P, C.POINTER(C.c_double), _SZ, C.POINTER(C.c_double)]),
+    "msb_state_hp_gibbs": (C.c_int, [_P, C.POINTER(HpGibbsOpts), C.POINTER(HpGibbsOut)]),
     "msb_state_delta_buffer": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),
     "msb_state_apply_deltas": (C.c_int, [_P]),
     "msb_state_delta_buffer_i32": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),

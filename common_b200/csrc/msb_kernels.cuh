@@ -602,22 +602,20 @@ __global__ void niw_prepare_kernel(FeatDev f, const double *__restrict__ hp, con
 // ---------------------------------------------------------------------------
 __device__ __forceinline__ double lbeta_d(double a, double b) { return lgamma(a) + lgamma(b) - lgamma(a + b); }
 
-__global__ void score_data_kernel(const FeatDev *__restrict__ feats, int nfeat, const double *__restrict__ hp,
-                                  const double *__restrict__ ss, const int32_t *__restrict__ col2slot, int ncols,
-                                  double *__restrict__ out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= ncols * nfeat) return;
-  const int col = i / nfeat, d = i - col * nfeat;
-  const FeatDev f = feats[d];
-  if (f.kind == KIND_NIW) return;  // niw_score_data_kernel
-  const double *h = hp + f.hp_off;
-  const double *g = ss + f.ss_off + (size_t)col2slot[col] * f.ss_w;
+// The closed form of one (group, feature) cell, every family but niw: h = the feature's hp vector, asum = the dd alpha
+// sum that goes with h, g = the group's suffstats.  A dd / dm category with count 0 adds lgamma(a) - lgamma(a) = +0
+// exactly, so it is skipped: the result is the same bits as the full walk.
+__device__ __forceinline__ double score_data_cell(const FeatDev &f, const double *__restrict__ h, double asum,
+                                                  const double *__restrict__ g) {
   double r;
   if (f.family == FAM_DM) {  // dm.cpp:79-95; ss = [counts[dim], ratio]
-    double asum = 0.0, csum = 0.0;
+    double as = 0.0, csum = 0.0;
     r = g[f.dim];
-    for (uint32_t c = 0; c < f.dim; c++) { asum += h[c]; csum += g[c]; r += lgamma(g[c] + h[c]) - lgamma(h[c]); }
-    r += lgamma(asum) - lgamma(asum + csum);
+    for (uint32_t c = 0; c < f.dim; c++) {
+      as += h[c];
+      if (g[c] != 0.0) { csum += g[c]; r += lgamma(g[c] + h[c]) - lgamma(h[c]); }
+    }
+    r += lgamma(as) - lgamma(as + csum);
   } else if (f.family == FAM_BB) {
     r = lbeta_d(h[0] + g[0], h[1] + g[1]) - lbeta_d(h[0], h[1]);
   } else if (f.family == FAM_BBNC) {  // bbnc.cpp:61-73: Beta prior density of p + Bernoulli likelihood of the counts
@@ -625,8 +623,9 @@ __global__ void score_data_kernel(const FeatDev *__restrict__ feats, int nfeat, 
     r = (p < 0.0 || p > 1.0) ? -CUDART_INF
                              : (h[0] - 1.0) * log(p) + (h[1] - 1.0) * log1p(-p) - lbeta_d(h[0], h[1]) + g[1] * log(p) + g[2] * log1p(-p);
   } else if (f.family == FAM_DD) {
-    r = lgamma(f.asum) - lgamma(f.asum + g[0]);
-    for (uint32_t c = 0; c < f.dim; c++) r += lgamma(h[c] + g[1 + c]) - lgamma(h[c]);
+    r = lgamma(asum) - lgamma(asum + g[0]);
+    for (uint32_t c = 0; c < f.dim; c++)
+      if (g[1 + c] != 0.0) r += lgamma(h[c] + g[1 + c]) - lgamma(h[c]);
   } else if (f.family == FAM_BNB) {
     // (count, sum) do not determine sum_i [lgamma(r + x_i) - lgamma(r) - lgamma(x_i + 1)]: like the family's own
     // two-field group this returns the part that depends on the partition and on (alpha, beta)
@@ -646,7 +645,18 @@ __global__ void score_data_kernel(const FeatDev *__restrict__ feats, int nfeat, 
     r = lgamma(0.5 * nu) - lgamma(0.5 * h[3]) + 0.5 * log(h[1] / kappa) + 0.5 * h[3] * log(h[3] * h[2]) -
         0.5 * nu * log(nu * sigmasq) - 0.5 * n * log(CUDART_PI);
   }
-  out[i] = r;
+  return r;
+}
+
+__global__ void score_data_kernel(const FeatDev *__restrict__ feats, int nfeat, const double *__restrict__ hp,
+                                  const double *__restrict__ ss, const int32_t *__restrict__ col2slot, int ncols,
+                                  double *__restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= ncols * nfeat) return;
+  const int col = i / nfeat, d = i - col * nfeat;
+  const FeatDev f = feats[d];
+  if (f.kind == KIND_NIW) return;  // niw_score_data_kernel
+  out[i] = score_data_cell(f, hp + f.hp_off, f.asum, ss + f.ss_off + (size_t)col2slot[col] * f.ss_w);
 }
 
 // In-place lower Cholesky of the d x d matrix A in shared memory by the whole block (right-looking, as in

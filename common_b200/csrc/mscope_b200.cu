@@ -23,6 +23,7 @@
 #include "msb_niw_tc16.cuh"
 #include "msb_draw.cuh"
 #include "msb_predict.cuh"
+#include "msb_hp.cuh"
 
 using namespace msb;
 
@@ -192,6 +193,13 @@ struct msb_state {
   size_t ring_nchunks[TIMING_RING] = {0};
   uint64_t sweep_seq = 0;  // sweeps enqueued so far
   size_t last_allreduce_bytes = 0;  // message size of the last msb_state_allreduce_deltas
+  // hyperparameter grids (msb_state_set_hp_grid / set_cluster_hp_grid): [D + 1] host copies, row D = alpha's; the device
+  // buffer d_grid = [HpRow rows | points | log priors] is rebuilt whenever a grid is set
+  std::vector<std::vector<double>> grid_pts, grid_lp;
+  std::vector<HpRow> hp_rows;
+  size_t grid_gmax = 0;
+  void *d_grid = nullptr;
+  double *d_hpwork = nullptr; size_t hpwork_cap = 0;  // msb_state_hp_gibbs scratch
 };
 
 #define LAUNCH(ctx, kernel, grid, block, smem, ...)                      \
@@ -726,6 +734,7 @@ extern "C" MSB_API int msb_state_destroy(msb_state *st) {
   for (size_t d = 0; d < st->D; d++) { cudaFree(st->d_niwW[d]); cudaFree(st->d_niwBias[d]); cudaFree(st->d_niwCoef[d]); cudaFree(st->d_niwB[d]); }
   cudaFree(st->d_niwA16);
   cudaFree(st->d_rowmax);
+  cudaFree(st->d_grid); cudaFree(st->d_hpwork);
   cudaFree(st->d_feats); cudaFree(st->d_feats_scalar); cudaFree(st->d_hp); cudaFree(st->d_ss); cudaFree(st->d_delta); cudaFree(st->d_delta_i32); cudaFree(st->d_counter);
   cudaFree(st->d_slot2gid); cudaFree(st->d_assign64); cudaFree(st->d_flags); cudaFreeHost(st->h_moved); cudaFreeHost(st->h_flags); cudaFree(st->d_assign); cudaFree(st->d_params); cudaFree(st->d_scores);
   cudaFree(st->d_base); cudaFree(st->d_base_score); cudaFree(st->d_col2slot); cudaFree(st->d_newslot); cudaFree(st->d_newcol); cudaFree(st->d_uniforms);
@@ -1146,12 +1155,8 @@ extern "C" MSB_API int msb_state_prefetch(msb_state *st) {
 }
 
 // ---- hypers / suffstats ------------------------------------------------------
-extern "C" MSB_API int msb_state_set_hp(msb_state *st, size_t feature, const char *key, const double *v, size_t count) {
-  REQUIRE(st && key && v, "NULL argument");
-  REQUIRE(feature < st->D, "bad feature index");
-  size_t off, cnt;
-  MSB_TRY(hp_field(st->models[feature], key, &off, &cnt));
-  REQUIRE(count == cnt, "wrong dimension");  // distributions.hpp:436
+// h_hp[feature][off, off + cnt) = v, and what follows the hypers: dd's alpha sum in both feature tables, the uploads
+static void write_hp(msb_state *st, size_t feature, size_t off, const double *v, size_t cnt) {
   double *h = st->h_hp.data() + st->feats[feature].hp_off;
   for (size_t i = 0; i < cnt; i++) h[off + i] = v[i];
   if (st->models[feature].family == MSB_FAMILY_DD) {
@@ -1162,6 +1167,14 @@ extern "C" MSB_API int msb_state_set_hp(msb_state *st, size_t feature, const cha
     st->feats_dirty = true;
   }
   st->hp_dirty = true;
+}
+extern "C" MSB_API int msb_state_set_hp(msb_state *st, size_t feature, const char *key, const double *v, size_t count) {
+  REQUIRE(st && key && v, "NULL argument");
+  REQUIRE(feature < st->D, "bad feature index");
+  size_t off, cnt;
+  MSB_TRY(hp_field(st->models[feature], key, &off, &cnt));
+  REQUIRE(count == cnt, "wrong dimension");  // distributions.hpp:436
+  write_hp(st, feature, off, v, cnt);
   return MSB_OK;
 }
 extern "C" MSB_API int msb_state_get_hp(msb_state *st, size_t feature, const char *key, double *v, size_t count) {
@@ -2673,6 +2686,183 @@ extern "C" MSB_API int msb_state_predict(msb_state *st, size_t row_lo, size_t ro
     uint32_t bad = 0;
     CU_TRY(cudaMemcpy(&bad, d_unsupported, sizeof(bad), cudaMemcpyDeviceToHost));
     if (bad) return fail(MSB_ERR_UNSUPPORTED, "multinomial sampling unimplemented");  // dm.cpp:100-111
+  }
+  return MSB_OK;
+}
+
+// ---- hyperparameter grids: one Gibbs step over the hypers (DESIGN.md section 4.10) ------------------------------------
+// bnb's score_data drops the r-dependent data term (score_data_cell), so the conditional of a grid over r is not the
+// one these weights give: every point must carry the feature's current r
+static int check_bnb_r(const msb_state *st, size_t feature, const double *pts, size_t npoints) {
+  const double r = st->h_hp[st->feats[feature].hp_off + 2];
+  for (size_t g = 0; g < npoints; g++)
+    if (pts[g * 3 + 2] != r)
+      return fail(MSB_ERR_INVALID, "feature " + std::to_string(feature) + ": bnb grid point " + std::to_string(g) +
+                                       " changes r; only (alpha, beta) can be resampled on a grid");
+  return MSB_OK;
+}
+
+static int upload_grids(msb_state *st) {
+  std::vector<HpRow> rows;
+  size_t npts = 0, nlp = 0, gmax = 0;
+  for (size_t d = 0; d <= st->D; d++) {
+    const size_t G = st->grid_lp[d].size();
+    if (!G) continue;
+    HpRow r;
+    memset(&r, 0, sizeof(r));
+    r.feat = (int32_t)d; r.npoints = (int32_t)G; r.nhp = (uint32_t)(st->grid_pts[d].size() / G);
+    r.pt_off = npts; r.lp_off = nlp;
+    npts += st->grid_pts[d].size(); nlp += G; gmax = std::max(gmax, G);
+    rows.push_back(r);
+  }
+  const size_t rows_b = (sizeof(HpRow) * rows.size() + 255) / 256 * 256;
+  std::vector<char> h(rows_b + sizeof(double) * (npts + nlp));
+  if (!rows.empty()) memcpy(h.data(), rows.data(), sizeof(HpRow) * rows.size());
+  double *pts = (double *)(h.data() + rows_b), *lp = pts + npts;
+  for (const HpRow &r : rows) {
+    memcpy(pts + r.pt_off, st->grid_pts[r.feat].data(), sizeof(double) * st->grid_pts[r.feat].size());
+    memcpy(lp + r.lp_off, st->grid_lp[r.feat].data(), sizeof(double) * r.npoints);
+  }
+  CU_TRY(cudaSetDevice(st->ctx->device));
+  void *d = nullptr;
+  if (!rows.empty()) {
+    CU_TRY(cudaMalloc(&d, h.size()));
+    cudaError_t e = cudaMemcpyAsync(d, h.data(), h.size(), cudaMemcpyHostToDevice, st->ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st->ctx->stream);  // h is pageable and goes out of scope
+    if (e != cudaSuccess) { cudaFree(d); CU_TRY(e); }
+  }
+  CU_TRY(cudaStreamSynchronize(st->ctx->stream));  // an hp_gibbs still in flight may read the old buffer
+  CU_TRY(cudaFree(st->d_grid));
+  st->d_grid = d;
+  st->hp_rows = rows;
+  st->grid_gmax = gmax;
+  return MSB_OK;
+}
+
+static void grids_resize(msb_state *st) {
+  if (st->grid_lp.empty()) { st->grid_pts.resize(st->D + 1); st->grid_lp.resize(st->D + 1); }
+}
+
+// grid `row` (a feature, or D for alpha) := (pts, lp); the host copies change only if the device buffer was rebuilt
+static int replace_grid(msb_state *st, size_t row, std::vector<double> pts, std::vector<double> lp) {
+  st->grid_pts[row].swap(pts);
+  st->grid_lp[row].swap(lp);
+  const int rc = upload_grids(st);
+  if (rc != MSB_OK) { st->grid_pts[row].swap(pts); st->grid_lp[row].swap(lp); }
+  return rc;
+}
+
+// a grid's points are a launch dimension of the hp kernels (gridDim.y)
+constexpr size_t HP_MAX_POINTS = 65535;
+
+extern "C" MSB_API int msb_state_set_hp_grid(msb_state *st, size_t feature, const double *points, size_t npoints, size_t nhp,
+                                             const double *log_prior) {
+  REQUIRE(st, "NULL argument");
+  REQUIRE(feature < st->D, "bad feature index");
+  grids_resize(st);
+  if (npoints == 0) return replace_grid(st, feature, {}, {});
+  REQUIRE(points && log_prior, "NULL argument");
+  const msb_model_desc &m = st->models[feature];
+  REQUIRE(nhp == hp_size(m), "feature " + std::to_string(feature) + ": a grid point has " + std::to_string(nhp) +
+                                 " values, the family takes " + std::to_string(hp_size(m)));
+  REQUIRE(npoints <= HP_MAX_POINTS, "too many grid points: at most " + std::to_string(HP_MAX_POINTS));
+  for (size_t i = 0; i < npoints * nhp; i++) REQUIRE(std::isfinite(points[i]), "non-finite grid value");
+  for (size_t g = 0; g < npoints; g++) REQUIRE(std::isfinite(log_prior[g]), "non-finite log prior");
+  if (m.family == MSB_FAMILY_BNB) MSB_TRY(check_bnb_r(st, feature, points, npoints));
+  return replace_grid(st, feature, std::vector<double>(points, points + npoints * nhp),
+                      std::vector<double>(log_prior, log_prior + npoints));
+}
+
+extern "C" MSB_API int msb_state_set_cluster_hp_grid(msb_state *st, const double *alphas, size_t npoints, const double *log_prior) {
+  REQUIRE(st, "NULL argument");
+  grids_resize(st);
+  if (npoints == 0) return replace_grid(st, st->D, {}, {});
+  REQUIRE(alphas && log_prior, "NULL argument");
+  REQUIRE(npoints <= HP_MAX_POINTS, "too many grid points: at most " + std::to_string(HP_MAX_POINTS));
+  for (size_t g = 0; g < npoints; g++) {
+    REQUIRE(std::isfinite(alphas[g]) && alphas[g] > 0.0, "alpha must be positive and finite");  // group_manager.hpp:120
+    REQUIRE(std::isfinite(log_prior[g]), "non-finite log prior");
+  }
+  return replace_grid(st, st->D, std::vector<double>(alphas, alphas + npoints), std::vector<double>(log_prior, log_prior + npoints));
+}
+
+extern "C" MSB_API int msb_state_hp_gibbs(msb_state *st, const msb_hp_gibbs_opts *opts, msb_hp_gibbs_out *out) {
+  REQUIRE(st && opts, "NULL argument");
+  REQUIRE(opts->counter < (1ull << 32), "counter must be below 2^32");
+  const size_t D = st->D, R = st->hp_rows.size(), G = st->grid_gmax;
+  REQUIRE(!out || !out->logw || out->logw_ld >= G, "logw_ld smaller than the largest grid");
+  if (out && out->choice)
+    for (size_t d = 0; d <= D; d++) out->choice[d] = -1;
+  if (!R) return MSB_OK;
+  for (const HpRow &r : st->hp_rows)
+    if ((size_t)r.feat < D && st->models[r.feat].family == MSB_FAMILY_BNB)
+      MSB_TRY(check_bnb_r(st, r.feat, st->grid_pts[r.feat].data(), r.npoints));
+  msb_ctx *ctx = st->ctx;
+  CU_TRY(cudaSetDevice(ctx->device));
+  MSB_TRY(prepare_columns(st));
+  MSB_TRY(sync_small(st));
+  const size_t K = st->h_col2slot.size();
+  const size_t rows_b = (sizeof(HpRow) * R + 255) / 256 * 256;
+  const HpRow *d_rows = (const HpRow *)st->d_grid;
+  const double *d_pts = (const double *)((const char *)st->d_grid + rows_b);
+  size_t npts = 0;
+  for (const HpRow &r : st->hp_rows) npts += (size_t)r.npoints * r.nhp;
+  const double *d_lp = d_pts + npts;
+  // scratch: L [R][G] | logw [R][G] | choice [R] (int64) | niw, for the largest niw grid of P points: ld0 [P] and the
+  // per-(point, group) values [P][K]
+  size_t niw_pts = 0;
+  for (const HpRow &r : st->hp_rows)
+    if ((size_t)r.feat < D && st->feats[r.feat].kind == KIND_NIW) niw_pts = std::max(niw_pts, (size_t)r.npoints);
+  MSB_TRY(ensure(&st->d_hpwork, &st->hpwork_cap, 2 * R * G + R + niw_pts * (K + 1)));
+  double *d_L = st->d_hpwork, *d_logw = d_L + R * G;
+  int64_t *d_choice = (int64_t *)(d_logw + R * G);
+  double *d_ld0 = (double *)(d_choice + R), *d_niw = d_ld0 + niw_pts;
+  LAUNCH(ctx, hp_grid_kernel, dim3((unsigned)R, (unsigned)G), HP_THREADS, 0, st->d_feats, (int)D, d_rows, d_pts, st->d_ss,
+         st->d_col2slot, (int)K, G, d_L);
+  for (size_t i = 0; i < R; i++) {
+    const HpRow &r = st->hp_rows[i];
+    const double *pts = d_pts + r.pt_off;
+    if ((size_t)r.feat == D) {
+      LAUNCH(ctx, hp_alpha_kernel, 1, HP_THREADS, 0, st->d_ss, st->d_col2slot, (int)K, pts, r.npoints, d_L + i * G);
+      continue;
+    }
+    const FeatDev &f = st->feats[r.feat];
+    if (f.kind != KIND_NIW) continue;
+    const size_t smem0 = (size_t)f.dim * f.dim * sizeof(double), smem = smem0 + f.dim * sizeof(double);
+    if (smem > 48 * 1024) {
+      CU_TRY(opt_in_smem(niw_hp_prior_kernel, smem0));
+      CU_TRY(opt_in_smem(niw_hp_group_kernel, smem));
+    }
+    LAUNCH(ctx, niw_hp_prior_kernel, (unsigned)r.npoints, 128, smem0, (int)f.dim, pts, r.nhp, d_ld0);
+    LAUNCH(ctx, niw_hp_group_kernel, dim3((unsigned)K, (unsigned)r.npoints), 128, smem, f, pts, r.nhp, d_ld0, st->d_ss,
+           st->d_col2slot, (int)K, d_niw);
+    LAUNCH(ctx, hp_reduce_kernel, (unsigned)r.npoints, HP_THREADS, 0, d_niw, (int)K, d_L + i * G);
+  }
+  LAUNCH(ctx, hp_draw_kernel, cdiv(R, 32), 32, 0, d_rows, (int)R, d_lp, d_L, G, opts->seed, opts->counter, d_logw, d_choice);
+  std::vector<double> h(R * G + R);
+  CU_TRY(cudaMemcpyAsync(h.data(), d_logw, sizeof(double) * h.size(), cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(cudaStreamSynchronize(ctx->stream));
+  const double *logw = h.data();
+  const int64_t *choice = (const int64_t *)(h.data() + R * G);
+  for (size_t i = 0; i < R; i++) {
+    if (choice[i] >= 0) continue;
+    const HpRow &r = st->hp_rows[i];
+    const std::string who = (size_t)r.feat == D ? std::string("alpha") : "feature " + std::to_string(r.feat);
+    for (int g = 0; g < r.npoints; g++) {
+      const double w = logw[i * G + g];
+      if (std::isnan(w)) return fail(MSB_ERR_INVALID, who + ": grid point " + std::to_string(g) + " has a NaN weight");
+      if (w == HUGE_VAL) return fail(MSB_ERR_INVALID, who + ": grid point " + std::to_string(g) + " has weight +inf");
+    }
+    return fail(MSB_ERR_INVALID, who + ": every grid point has weight -inf");
+  }
+  for (size_t i = 0; i < R; i++) {
+    const HpRow &r = st->hp_rows[i];
+    const double *pt = st->grid_pts[r.feat].data() + (size_t)choice[i] * r.nhp;
+    if ((size_t)r.feat == D) st->alpha = *pt;
+    else write_hp(st, r.feat, 0, pt, r.nhp);
+    if (out && out->choice) out->choice[r.feat] = choice[i];
+    if (out && out->logw)
+      for (int g = 0; g < r.npoints; g++) out->logw[(size_t)r.feat * out->logw_ld + g] = logw[i * G + g];
   }
   return MSB_OK;
 }

@@ -17,6 +17,12 @@ def _dbl(values):
     return a, a.ctypes.data_as(C.POINTER(C.c_double))
 
 
+def flat_hp(model, hp):
+    """one hp dict with the keys of model.default_hyperparams() as the flat vector of the C ABI (include/mscope_b200.h,
+    enum msb_family): the values in that key order"""
+    return np.concatenate([np.asarray(hp[k], np.float64).ravel() for k in model.default_hyperparams()])
+
+
 class state(object):
     def __init__(self, ctx, models, max_groups=64, cluster_hp=None):
         self._ctx = ctx
@@ -26,6 +32,7 @@ class state(object):
         _lib.check(_lib.load().msb_state_create(ctx.handle, descs, len(self._models), int(max_groups), C.byref(h)))
         self._h = h
         self._view = None
+        self._grid_sizes = {}     # component (or "alpha") -> number of grid points registered
         ctx._adopt(self)
         if cluster_hp is not None:
             self.set_cluster_hp(cluster_hp)
@@ -80,6 +87,56 @@ class state(object):
     def set_hp_raw(self, component, key, values):
         a, p = _dbl(values)
         _lib.check(_lib.load().msb_state_set_hp(self._h, component, key.encode(), p, a.size))
+
+    # ---- hyperparameter inference on a grid (msb_state_hp_gibbs) ------------------------------------------------
+    def set_hp_grid(self, component, points, log_prior=None):
+        """register a grid for the component's hypers: ``points`` a list of hp dicts, ``log_prior`` the caller's log
+        hyperprior at each point (default: uniform).  points=None removes the grid"""
+        lib = _lib.load()
+        if points is None or len(points) == 0:
+            _lib.check(lib.msb_state_set_hp_grid(self._h, component, None, 0, 0, None))
+            self._grid_sizes.pop(component, None)
+            return
+        flat = np.stack([flat_hp(self._models[component], p) for p in points])
+        a, pa = _dbl(flat)
+        lp, plp = _dbl(np.zeros(len(points)) if log_prior is None else log_prior)
+        if lp.size != len(points):
+            raise ValueError("one log prior per grid point: %d points, %d log priors" % (len(points), lp.size))
+        _lib.check(lib.msb_state_set_hp_grid(self._h, component, pa, flat.shape[0], flat.shape[1], plp))
+        self._grid_sizes[component] = flat.shape[0]
+
+    def set_cluster_hp_grid(self, alphas, log_prior=None):
+        """register a grid for the CRP concentration; alphas=None removes it"""
+        lib = _lib.load()
+        if alphas is None or len(alphas) == 0:
+            _lib.check(lib.msb_state_set_cluster_hp_grid(self._h, None, 0, None))
+            self._grid_sizes.pop("alpha", None)
+            return
+        a, pa = _dbl(alphas)
+        lp, plp = _dbl(np.zeros(a.size) if log_prior is None else log_prior)
+        if lp.size != a.size:
+            raise ValueError("one log prior per grid point: %d points, %d log priors" % (a.size, lp.size))
+        _lib.check(lib.msb_state_set_cluster_hp_grid(self._h, pa, a.size, plp))
+        self._grid_sizes["alpha"] = a.size
+
+    def hp_gibbs(self, seed=0, counter=0, weights=False):
+        """one Gibbs step over every registered grid (features and alpha), drawn on the device and applied to the state.
+        Returns {"choice": {component: index, ..., "alpha": index}} for the grids that exist, and with weights=True
+        also "logw": {same keys: float64 array of log_prior + log marginal per point}"""
+        D = len(self._models)
+        choice = np.full(D + 1, -1, np.int64)
+        out = _lib.HpGibbsOut(choice.ctypes.data, None, 0)
+        logw = None
+        if weights:
+            logw = np.zeros((D + 1, max(self._grid_sizes.values(), default=1)))
+            out.logw, out.logw_ld = logw.ctypes.data, logw.shape[1]
+        opts = _lib.HpGibbsOpts(int(seed), int(counter))
+        _lib.check(_lib.load().msb_state_hp_gibbs(self._h, C.byref(opts), C.byref(out)))
+        keys = list(range(D)) + ["alpha"]
+        res = {"choice": {keys[d]: int(choice[d]) for d in range(D + 1) if choice[d] >= 0}}
+        if weights:
+            res["logw"] = {k: logw[d][:self._grid_sizes[k]].copy() for d, k in enumerate(keys) if choice[d] >= 0}
+        return res
 
     # ---- suffstats (entity_state.hpp:51-54) --------------------------------------
     def get_suffstats(self, component, gid, key, count=1):

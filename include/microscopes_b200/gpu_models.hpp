@@ -15,6 +15,8 @@
 // Header-only; link with -lmscope_b200.
 #pragma once
 
+#include <algorithm>
+#include <cstring>
 #include <map>
 #include <sstream>
 
@@ -313,6 +315,37 @@ public:
     if (gids) *gids = g;
     return logp;
   }
+  // hyperparameter grids (msb_state_set_hp_grid / set_cluster_hp_grid): points[npoints][nhp] in the flat hp layout,
+  // log_prior[npoints]; an empty grid removes it
+  void set_hp_grid(size_t feature, const std::vector<double> &points, const std::vector<double> &log_prior) {
+    const size_t g = log_prior.size();
+    b200::check(msb_state_set_hp_grid(st_, feature, points.data(), g, g ? points.size() / g : 0, log_prior.data()));
+    grid_sizes_[feature] = g;
+  }
+  void set_cluster_hp_grid(const std::vector<double> &alphas, const std::vector<double> &log_prior) {
+    b200::check(msb_state_set_cluster_hp_grid(st_, alphas.data(), alphas.size(), log_prior.data()));
+    grid_sizes_[D_] = alphas.size();
+  }
+  // one Gibbs step over every grid (msb_state_hp_gibbs), applied to the state: the index drawn per feature, -1 without a
+  // grid, [D] = alpha's; logw ([D + 1][*logw_ld], log_prior + log marginal per point) when the pointer is non-null
+  std::vector<int64_t> hp_gibbs(uint64_t seed, uint64_t counter, std::vector<double> *logw = nullptr,
+                                size_t *logw_ld = nullptr) {
+    std::vector<int64_t> choice(D_ + 1, -1);
+    msb_hp_gibbs_opts o;
+    o.seed = seed; o.counter = counter;
+    msb_hp_gibbs_out out;
+    std::memset(&out, 0, sizeof(out));
+    out.choice = choice.data();
+    if (logw) {
+      size_t ld = 1;
+      for (const auto &g : grid_sizes_) ld = std::max(ld, g.second);
+      logw->assign((D_ + 1) * ld, 0.0);
+      out.logw = logw->data(); out.logw_ld = ld;
+      if (logw_ld) *logw_ld = ld;
+    }
+    b200::check(msb_state_hp_gibbs(st_, &o, &out));
+    return choice;
+  }
   msb_sweep_result sweep(uint64_t seed, uint64_t sweep_id) {
     msb_sweep_opts o;
     std::memset(&o, 0, sizeof(o));
@@ -366,6 +399,7 @@ private:
   msb_state *st_;
   size_t D_;
   std::vector<msb_model_desc> descs_;
+  std::map<size_t, size_t> grid_sizes_;  // feature (D_: alpha) -> grid points registered
 };
 
 }  // namespace models

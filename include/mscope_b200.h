@@ -29,6 +29,7 @@
  *                         (SURVEY.md section 3b) against frozen suffstats
  *   msb_state_predict     mixturemodel's score_value (logsumexp of one inplace_score_value over the groups), the
  *                         responsibilities, and sample_post_pred's imputation of masked cells, for a row range
+ *   msb_state_hp_gibbs    mixturemodel's grid feature-hp and cluster-hp kernels: one Gibbs step over gridded hypers
  *   msb_value_*           single-value group::score_value/add_value/remove_value/score_data/sample_value
  *                         (models/base.hpp:25-27), executed on the device
  *
@@ -313,6 +314,45 @@ typedef struct msb_predict_out {      /* host pointers; NULL = not wanted */
 } msb_predict_out;
 MSB_API int msb_state_predict(msb_state *st, size_t row_lo, size_t row_hi, const msb_predict_opts *opts,
                               msb_predict_out *out, size_t *gids, size_t cap, size_t *ncols);
+
+/* ---- hyperparameter inference on a grid (DESIGN.md section 4.10) -----------------------------------------------------
+ * The mixturemodel runner's grid feature-hp kernel and its cluster-hp kernel, on the device.  Grids are registered once
+ * and stay resident; the caller supplies the log hyperprior of every point (the library evaluates no hyperprior density).
+ *
+ * msb_state_set_hp_grid: feature `feature` gets npoints >= 1 grid points, each a complete hp vector in the flat layout
+ * msb_value_score_data takes (nhp doubles; bb: alpha, beta; bnb: alpha, beta, r; gp: alpha, inv_beta; nich: mu, kappa,
+ * sigmasq, nu; dd / dm: alphas[C]; niw: mu[d], kappa, psi[d*d], nu; bbnc: alpha, beta), points[npoints][nhp] row-major,
+ * log_prior[npoints].  npoints == 0 removes the feature's grid.  msb_state_set_cluster_hp_grid: the same for the CRP
+ * concentration, alphas[npoints] > 0.  A grid holds at most 65535 points.
+ * Refused with MSB_ERR_INVALID, the state untouched: nhp that is not the family's, a non-finite value or log prior, an
+ * alpha <= 0, more than 65535 points, a bnb point whose r differs from the feature's current r (bnb's score_data drops the r-dependent data
+ * term, so only (alpha, beta) can be resampled).
+ *
+ * msb_state_hp_gibbs: one Gibbs step for every feature that has a grid, and for alpha if it has one.
+ *   feature d:  L[g] = sum over every group column (ascending gid, empty groups included) of score_data(theta_g), fp64
+ *               -- the set msb_state_score_likelihood_all sums, nothing rounded to float
+ *   alpha:      L[g] = (#non-empty groups - 1) log alpha_g + lgamma(1 + alpha_g) - lgamma(n + alpha_g), n = assigned entities
+ *   w_g = log_prior[g] + L[g], m = max w, p_g = exp(w_g - m) summed in index order in fp64; the draw is the first g whose
+ *   running sum exceeds u * sum p, u a 53-bit uniform from philox4x32_10(key = seed, counter = (d, HP_TAG | counter))
+ *   (alpha: d = D; its two first words a, b give u = ((a >> 5) 2^26 + (b >> 6)) 2^-53).  counter >= 2^32: MSB_ERR_INVALID.
+ *   The sums over groups have a fixed order and no atomics: identical suffstats give identical weights and draws, so
+ *   replicas after msb_state_allreduce_deltas draw the same hypers without a collective.
+ *   The drawn points are written as msb_state_set_hp / msb_state_set_cluster_hp write them; assignments, suffstats,
+ *   deltas and the sweep timing ring do not change.  Pending deferred deltas are not included (as for score_likelihood).
+ *   A NaN or +inf weight (e.g. a niw psi that is not positive definite) or a grid whose weights are all -inf: MSB_ERR_INVALID,
+ *   naming the feature and the point, and no hyper is changed.
+ *   out (host pointers, each may be NULL): choice[D + 1] = the index drawn per feature, -1 without a grid, [D] = alpha's;
+ *   logw[(D + 1) * logw_ld], logw_ld >= the largest grid: row d holds w_g of feature d (row D: alpha); rows without a
+ *   grid are not written. */
+MSB_API int msb_state_set_hp_grid(msb_state *st, size_t feature, const double *points, size_t npoints, size_t nhp,
+                                  const double *log_prior);
+MSB_API int msb_state_set_cluster_hp_grid(msb_state *st, const double *alphas, size_t npoints, const double *log_prior);
+typedef struct msb_hp_gibbs_opts { uint64_t seed, counter; } msb_hp_gibbs_opts;
+typedef struct msb_hp_gibbs_out {     /* host pointers; NULL = not wanted */
+  int64_t *choice;                    /* [D + 1] */
+  double *logw; size_t logw_ld;       /* [D + 1][logw_ld] */
+} msb_hp_gibbs_out;
+MSB_API int msb_state_hp_gibbs(msb_state *st, const msb_hp_gibbs_opts *opts, msb_hp_gibbs_out *out);
 
 /* multi-GPU: flat fp64 buffer [group counts | per-feature suffstat deltas] on the device */
 MSB_API int msb_state_delta_buffer(msb_state *st, double **dev_ptr, size_t *count);
