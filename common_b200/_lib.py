@@ -73,6 +73,14 @@ class HpGibbsOut(C.Structure):
     _fields_ = [("choice", C.c_void_p), ("logw", C.c_void_p), ("logw_ld", C.c_size_t)]
 
 
+class ThetaOpts(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("counter", C.c_uint64), ("widths", C.c_void_p), ("nwidths", C.c_size_t)]
+
+
+class ThetaOut(C.Structure):
+    _fields_ = [("capped", C.c_size_t)]
+
+
 _P = C.c_void_p
 _SZ = C.c_size_t
 _PROTOS = {
@@ -141,6 +149,8 @@ _PROTOS = {
     "msb_state_set_hp_grid": (C.c_int, [_P, _SZ, C.POINTER(C.c_double), _SZ, _SZ, C.POINTER(C.c_double)]),
     "msb_state_set_cluster_hp_grid": (C.c_int, [_P, C.POINTER(C.c_double), _SZ, C.POINTER(C.c_double)]),
     "msb_state_hp_gibbs": (C.c_int, [_P, C.POINTER(HpGibbsOpts), C.POINTER(HpGibbsOut)]),
+    "msb_state_theta": (C.c_int, [_P, C.POINTER(ThetaOpts), C.POINTER(ThetaOut)]),
+    "msb_state_redraw_empty": (C.c_int, [_P, C.c_uint64, C.c_uint64]),
     "msb_state_delta_buffer": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),
     "msb_state_apply_deltas": (C.c_int, [_P]),
     "msb_state_delta_buffer_i32": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),

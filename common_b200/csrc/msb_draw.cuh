@@ -18,13 +18,14 @@ namespace msb {
 constexpr uint64_t DRAW_TAG = 0x53414d5000000000ull;  // "SAMP": keeps these counters apart from the sweeps' (row, sweep) ones
 constexpr uint32_t DRAW_WALK_CAP = 1u << 26;          // longest pmf walk of the count families (bnb has no mean for a <= 1)
 
+// block b of the stream is philox4x32_10(seed, idx, tag | b); other callers (msb_theta.cuh) pass their own tag
 struct DrawStream {
-  uint64_t seed, idx;
+  uint64_t seed, idx, tag;
   uint32_t blk, buf[4];
   int pos;
-  __device__ DrawStream(uint64_t s, uint64_t i) : seed(s), idx(i), blk(0), pos(4) {}
+  __device__ DrawStream(uint64_t s, uint64_t i, uint64_t t = DRAW_TAG) : seed(s), idx(i), tag(t), blk(0), pos(4) {}
   __device__ uint32_t next() {
-    if (pos == 4) { philox4x32_10(seed, idx, DRAW_TAG | blk, buf); blk++; pos = 0; }
+    if (pos == 4) { philox4x32_10(seed, idx, tag | blk, buf); blk++; pos = 0; }
     return buf[pos++];
   }
   __device__ double u53() {  // [0, 1), 53 bits

@@ -24,6 +24,7 @@
 #include "msb_draw.cuh"
 #include "msb_predict.cuh"
 #include "msb_hp.cuh"
+#include "msb_theta.cuh"
 
 using namespace msb;
 
@@ -200,6 +201,7 @@ struct msb_state {
   size_t grid_gmax = 0;
   void *d_grid = nullptr;
   double *d_hpwork = nullptr; size_t hpwork_cap = 0;  // msb_state_hp_gibbs scratch
+  char *d_theta = nullptr; size_t theta_cap = 0;        // msb_state_theta / redraw_empty scratch (theta_run)
 };
 
 #define LAUNCH(ctx, kernel, grid, block, smem, ...)                      \
@@ -734,7 +736,7 @@ extern "C" MSB_API int msb_state_destroy(msb_state *st) {
   for (size_t d = 0; d < st->D; d++) { cudaFree(st->d_niwW[d]); cudaFree(st->d_niwBias[d]); cudaFree(st->d_niwCoef[d]); cudaFree(st->d_niwB[d]); }
   cudaFree(st->d_niwA16);
   cudaFree(st->d_rowmax);
-  cudaFree(st->d_grid); cudaFree(st->d_hpwork);
+  cudaFree(st->d_grid); cudaFree(st->d_hpwork); cudaFree(st->d_theta);
   cudaFree(st->d_feats); cudaFree(st->d_feats_scalar); cudaFree(st->d_hp); cudaFree(st->d_ss); cudaFree(st->d_delta); cudaFree(st->d_delta_i32); cudaFree(st->d_counter);
   cudaFree(st->d_slot2gid); cudaFree(st->d_assign64); cudaFree(st->d_flags); cudaFreeHost(st->h_moved); cudaFreeHost(st->h_flags); cudaFree(st->d_assign); cudaFree(st->d_params); cudaFree(st->d_scores);
   cudaFree(st->d_base); cudaFree(st->d_base_score); cudaFree(st->d_col2slot); cudaFree(st->d_newslot); cudaFree(st->d_newcol); cudaFree(st->d_uniforms);
@@ -2865,6 +2867,99 @@ extern "C" MSB_API int msb_state_hp_gibbs(msb_state *st, const msb_hp_gibbs_opts
       for (int g = 0; g < r.npoints; g++) out->logw[(size_t)r.feat * out->logw_ld + g] = logw[i * G + g];
   }
   return MSB_OK;
+}
+
+// ---- non-conjugate parameters: slice sampling of bbnc's p, fresh p for the empty groups (DESIGN.md section 4.11) ------
+// The stream packing (msb_theta.cuh) holds a feature index in 16 bits; a launch covers at most 65535 features (gridDim.y)
+constexpr size_t THETA_MAX_FEATURE = 65535;
+
+// One launch of theta_kernel (slice) or redraw_empty_kernel over the features in tf and every group column, then the
+// call's one synchronise; the new p are committed into d_ss only if no column was refused.
+// d_theta = [flags: 2 x u32 | pad | ThetaFeat[A] | gid per column, u32 [K] | pad | p [A][K] (fp64) | status [A][K] (u8)]
+static int theta_run(msb_state *st, bool slice, const std::vector<ThetaFeat> &tf, uint64_t seed, uint64_t counter, size_t *capped) {
+  if (capped) *capped = 0;
+  if (tf.empty() || st->gid2slot.empty()) return MSB_OK;
+  for (const auto &p : st->gid2slot)
+    REQUIRE(p.first < (1ull << 32), "gid " + std::to_string(p.first) + " does not fit the stream packing (gids below 2^32)");
+  msb_ctx *ctx = st->ctx;
+  CU_TRY(cudaSetDevice(ctx->device));
+  MSB_TRY(prepare_columns(st));
+  MSB_TRY(sync_small(st));
+  const size_t K = st->h_col2slot.size(), A = tf.size();
+  const size_t off_tf = 16, off_gid = off_tf + sizeof(ThetaFeat) * A, off_p = (off_gid + sizeof(uint32_t) * K + 7) / 8 * 8,
+               off_s = off_p + sizeof(double) * A * K;
+  std::vector<char> h(off_p, 0);
+  const uint32_t flags0[2] = {0u, UINT32_MAX};
+  memcpy(h.data(), flags0, sizeof(flags0));
+  memcpy(h.data() + off_tf, tf.data(), sizeof(ThetaFeat) * A);
+  uint32_t *hg = (uint32_t *)(h.data() + off_gid);
+  for (size_t c = 0; c < K; c++) hg[c] = (uint32_t)st->h_colgid[c];
+  MSB_TRY(ensure(&st->d_theta, &st->theta_cap, off_s + A * K));
+  char *d = st->d_theta;
+  uint32_t *d_flags = (uint32_t *)d;
+  const ThetaFeat *d_tf = (const ThetaFeat *)(d + off_tf);
+  const uint32_t *d_gid = (const uint32_t *)(d + off_gid);
+  double *d_p = (double *)(d + off_p);
+  uint8_t *d_s = (uint8_t *)(d + off_s);
+  CU_TRY(cudaMemcpyAsync(d, h.data(), h.size(), cudaMemcpyHostToDevice, ctx->stream));  // pageable: staged on return
+  const dim3 grid(cdiv(K, THETA_THREADS), (unsigned)A);
+  if (slice)
+    LAUNCH(ctx, theta_kernel, grid, THETA_THREADS, 0, st->d_feats, d_tf, st->d_hp, st->d_ss, st->d_col2slot, d_gid, (int)K, seed,
+           counter, d_p, d_s, d_flags);
+  else
+    LAUNCH(ctx, redraw_empty_kernel, grid, THETA_THREADS, 0, st->d_feats, d_tf, st->d_hp, st->d_ss, st->d_col2slot, d_gid, (int)K,
+           seed, counter, d_p, d_s, d_flags);
+  uint32_t hf[2];
+  CU_TRY(cudaMemcpyAsync(hf, d_flags, sizeof(hf), cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(cudaStreamSynchronize(ctx->stream));
+  if (hf[1] != UINT32_MAX) {
+    const size_t a = hf[1] / K, c = hf[1] % K;
+    const std::string who = "feature " + std::to_string(tf[a].feat) + ": gid " + std::to_string(st->h_colgid[c]);
+    return fail(MSB_ERR_INVALID, slice ? who + ": the current p has a non-finite score_data; the slice update needs a finite density there"
+                                       : who + ": the Beta(alpha, beta) draw of p underflowed (both gamma variates are 0)");
+  }
+  LAUNCH(ctx, theta_commit_kernel, grid, THETA_THREADS, 0, st->d_feats, d_tf, st->d_col2slot, (int)K, d_p, d_s, st->d_ss);
+  for (size_t c = 0; c < K; c++) st->slot_dirty[st->h_col2slot[c]] = 1;
+  if (capped) *capped = hf[0];
+  return MSB_OK;
+}
+
+extern "C" MSB_API int msb_state_theta(msb_state *st, const msb_theta_opts *opts, msb_theta_out *out) {
+  static const char *const family_names[] = {"bb", "bnb", "gp", "nich", "dd", "niw", "bbnc", "dm"};
+  REQUIRE(st && opts, "NULL argument");
+  REQUIRE(opts->nwidths == st->D, std::to_string(opts->nwidths) + " widths for a state of " + std::to_string(st->D) + " features");
+  REQUIRE(opts->widths || st->D == 0, "NULL argument");
+  REQUIRE(opts->counter < (1ull << 32), "counter must be below 2^32");
+  std::vector<ThetaFeat> tf;
+  for (size_t d = 0; d < st->D; d++) {
+    const double w = opts->widths[d];
+    REQUIRE(std::isfinite(w) && w >= 0.0, "feature " + std::to_string(d) + ": the slice width must be finite and non-negative");
+    if (w == 0.0) continue;
+    REQUIRE(st->models[d].family == MSB_FAMILY_BBNC, "feature " + std::to_string(d) + ": " + family_names[st->models[d].family] +
+                                                         " has no non-conjugate parameter (only bbnc's p is slice-sampled)");
+    REQUIRE(d < THETA_MAX_FEATURE, "feature " + std::to_string(d) + ": the index does not fit the stream packing (below 65535)");
+    ThetaFeat t;
+    t.feat = (int32_t)d; t.pad = 0; t.w = w;
+    tf.push_back(t);
+  }
+  size_t capped = 0;
+  MSB_TRY(theta_run(st, true, tf, opts->seed, opts->counter, &capped));
+  if (out) out->capped = capped;
+  return MSB_OK;
+}
+
+extern "C" MSB_API int msb_state_redraw_empty(msb_state *st, uint64_t seed, uint64_t counter) {
+  REQUIRE(st, "NULL argument");
+  REQUIRE(counter < (1ull << 32), "counter must be below 2^32");
+  std::vector<ThetaFeat> tf;
+  for (size_t d = 0; d < st->D; d++) {
+    if (st->models[d].family != MSB_FAMILY_BBNC) continue;
+    REQUIRE(d < THETA_MAX_FEATURE, "feature " + std::to_string(d) + ": the index does not fit the stream packing (below 65535)");
+    ThetaFeat t;
+    t.feat = (int32_t)d; t.pad = 0; t.w = 0.0;
+    tf.push_back(t);
+  }
+  return theta_run(st, false, tf, seed, counter, nullptr);
 }
 
 // ---- one pass over host rows in ONE call ---------------------------------------------------------------------------

@@ -138,6 +138,26 @@ class state(object):
             res["logw"] = {k: logw[d][:self._grid_sizes[k]].copy() for d, k in enumerate(keys) if choice[d] >= 0}
         return res
 
+    # ---- non-conjugate parameters (msb_state_theta / msb_state_redraw_empty) --------------------------------------
+    def theta(self, tparams, seed=0, counter=0):
+        """one slice-sampling update of every group's non-conjugate parameter, for the features in ``tparams``, the
+        runner's {component: {"p": width}} (bbnc is the one family with such a parameter).  Returns the number of
+        updates that reached the shrink cap and kept their value"""
+        widths = np.zeros(len(self._models))
+        for d, params in tparams.items():
+            for key, w in params.items():
+                if key != "p":
+                    raise ValueError("component %d: no non-conjugate parameter %r (bbnc's is 'p')" % (d, key))
+                widths[d] = w
+        out = _lib.ThetaOut()
+        opts = _lib.ThetaOpts(int(seed), int(counter), widths.ctypes.data, widths.size)
+        _lib.check(_lib.load().msb_state_theta(self._h, C.byref(opts), C.byref(out)))
+        return out.capped
+
+    def redraw_empty(self, seed=0, counter=0):
+        """every empty group's bbnc p drawn afresh from Beta(alpha, beta): the auxiliary groups of Neal's algorithm 8"""
+        _lib.check(_lib.load().msb_state_redraw_empty(self._h, int(seed), int(counter)))
+
     # ---- suffstats (entity_state.hpp:51-54) --------------------------------------
     def get_suffstats(self, component, gid, key, count=1):
         a = np.zeros(count, np.float64)

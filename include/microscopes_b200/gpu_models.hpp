@@ -346,6 +346,17 @@ public:
     b200::check(msb_state_hp_gibbs(st_, &o, &out));
     return choice;
   }
+  // one slice-sampling update of bbnc's p in every group (msb_state_theta): widths[D], 0 leaves a feature alone;
+  // returns the number of updates that reached the shrink cap and kept their p
+  size_t theta(const std::vector<double> &widths, uint64_t seed, uint64_t counter) {
+    msb_theta_opts o;
+    o.seed = seed; o.counter = counter; o.widths = widths.data(); o.nwidths = widths.size();
+    msb_theta_out out = {0};
+    b200::check(msb_state_theta(st_, &o, &out));
+    return out.capped;
+  }
+  // every empty group's bbnc p drawn afresh from Beta(alpha, beta) (msb_state_redraw_empty)
+  void redraw_empty(uint64_t seed, uint64_t counter) { b200::check(msb_state_redraw_empty(st_, seed, counter)); }
   msb_sweep_result sweep(uint64_t seed, uint64_t sweep_id) {
     msb_sweep_opts o;
     std::memset(&o, 0, sizeof(o));

@@ -30,6 +30,9 @@
  *   msb_state_predict     mixturemodel's score_value (logsumexp of one inplace_score_value over the groups), the
  *                         responsibilities, and sample_post_pred's imputation of masked cells, for a row range
  *   msb_state_hp_gibbs    mixturemodel's grid feature-hp and cluster-hp kernels: one Gibbs step over gridded hypers
+ *   msb_state_theta / redraw_empty
+ *                         mixturemodel's theta kernel (slice sampling of bbnc's p) and the auxiliary-parameter
+ *                         step of its assign_resample kernel (Neal's algorithm 8: the empty groups' p from the prior)
  *   msb_value_*           single-value group::score_value/add_value/remove_value/score_data/sample_value
  *                         (models/base.hpp:25-27), executed on the device
  *
@@ -353,6 +356,30 @@ typedef struct msb_hp_gibbs_out {     /* host pointers; NULL = not wanted */
   double *logw; size_t logw_ld;       /* [D + 1][logw_ld] */
 } msb_hp_gibbs_out;
 MSB_API int msb_state_hp_gibbs(msb_state *st, const msb_hp_gibbs_opts *opts, msb_hp_gibbs_out *out);
+
+/* ---- non-conjugate parameters (DESIGN.md section 4.11) ---------------------------------------------------------------
+ * msb_state_theta: one univariate slice-sampling update (Neal 2003: stepping out with width w, then shrinkage) of bbnc's
+ * p in every group column, empty groups included, for every feature whose width widths[d] > 0 (0 leaves the feature
+ * alone; nwidths must be D).  The target is the group's score_data with p substituted, the function
+ * msb_state_score_likelihood evaluates.  An update that reaches the cap of 200 shrink steps (or 2^20 stepping-out
+ * steps on a side) keeps its p and is counted in out->capped.  Draws come from
+ * philox4x32_10(key = seed, counter = (counter << 32 | gid, THETA_TAG | d << 16 | block)): identical suffstats give
+ * identical p, on every replica and after deserialisation.  Pending deferred deltas are not included.
+ * msb_state_redraw_empty: every bbnc feature's p of every group whose resident count is 0 becomes a fresh
+ * Beta(alpha, beta) draw x / (x + y) from the same packing under AUX_TAG; groups with members keep their p bit for bit.
+ * Without a bbnc feature it does nothing.
+ * Both write p into the suffstats (msb_state_get_ss "p") after the call's one synchronise, and only if no column was
+ * refused.  Refused with MSB_ERR_INVALID, the state untouched: a width that is negative or not finite, a width > 0 on a
+ * family other than bbnc, nwidths != D, counter >= 2^32, a feature index >= 65535 or a gid >= 2^32, a group whose
+ * current p has a non-finite score_data (e.g. p set to 0 or 1 by hand), a Beta draw that underflowed (the message names
+ * the feature and the gid). */
+typedef struct msb_theta_opts {
+  uint64_t seed, counter;
+  const double *widths; size_t nwidths;   /* [D] slice widths; 0 = leave the feature alone */
+} msb_theta_opts;
+typedef struct msb_theta_out { size_t capped; } msb_theta_out;
+MSB_API int msb_state_theta(msb_state *st, const msb_theta_opts *opts, msb_theta_out *out);
+MSB_API int msb_state_redraw_empty(msb_state *st, uint64_t seed, uint64_t counter);
 
 /* multi-GPU: flat fp64 buffer [group counts | per-feature suffstat deltas] on the device */
 MSB_API int msb_state_delta_buffer(msb_state *st, double **dev_ptr, size_t *count);
