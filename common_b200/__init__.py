@@ -12,7 +12,9 @@ from ._lib import Context, MsbError
 from .models import bb, bbnc, bnb, gp, nich, dd, dm, niw, model_descriptor
 from .dataview import numpy_dataview
 from .state import state, sample_discrete_log, philox_uniforms
+from .hyperprior import log_exponential, log_normal, log_flat, log_noninformative_beta_prior
 from . import synth
 
 __all__ = ["Context", "MsbError", "bb", "bbnc", "bnb", "gp", "nich", "dd", "dm", "niw", "model_descriptor",
-           "numpy_dataview", "state", "sample_discrete_log", "philox_uniforms"]
+           "numpy_dataview", "state", "sample_discrete_log", "philox_uniforms", "log_exponential", "log_normal", "log_flat",
+           "log_noninformative_beta_prior"]

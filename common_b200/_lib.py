@@ -81,6 +81,19 @@ class ThetaOut(C.Structure):
     _fields_ = [("capped", C.c_size_t)]
 
 
+class SliceHpSpec(C.Structure):
+    _fields_ = [("feature", C.c_size_t), ("key", C.c_char_p), ("width", C.c_double), ("prior", C.c_int32), ("a", C.c_double),
+                ("b", C.c_double)]
+
+
+class SliceHpOpts(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("counter", C.c_uint64), ("specs", C.POINTER(SliceHpSpec)), ("nspecs", C.c_size_t)]
+
+
+class SliceHpOut(C.Structure):
+    _fields_ = [("capped", C.c_size_t), ("values", C.c_void_p)]
+
+
 _P = C.c_void_p
 _SZ = C.c_size_t
 _PROTOS = {
@@ -151,6 +164,7 @@ _PROTOS = {
     "msb_state_hp_gibbs": (C.c_int, [_P, C.POINTER(HpGibbsOpts), C.POINTER(HpGibbsOut)]),
     "msb_state_theta": (C.c_int, [_P, C.POINTER(ThetaOpts), C.POINTER(ThetaOut)]),
     "msb_state_redraw_empty": (C.c_int, [_P, C.c_uint64, C.c_uint64]),
+    "msb_state_slice_hp": (C.c_int, [_P, C.POINTER(SliceHpOpts), C.POINTER(SliceHpOut)]),
     "msb_state_delta_buffer": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),
     "msb_state_apply_deltas": (C.c_int, [_P]),
     "msb_state_delta_buffer_i32": (C.c_int, [_P, C.POINTER(_P), C.POINTER(_SZ)]),

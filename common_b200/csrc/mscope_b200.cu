@@ -25,6 +25,7 @@
 #include "msb_predict.cuh"
 #include "msb_hp.cuh"
 #include "msb_theta.cuh"
+#include "msb_hpslice.cuh"
 
 using namespace msb;
 
@@ -202,6 +203,7 @@ struct msb_state {
   void *d_grid = nullptr;
   double *d_hpwork = nullptr; size_t hpwork_cap = 0;  // msb_state_hp_gibbs scratch
   char *d_theta = nullptr; size_t theta_cap = 0;        // msb_state_theta / redraw_empty scratch (theta_run)
+  char *d_hpsl = nullptr; size_t hpsl_cap = 0;          // msb_state_slice_hp scratch
 };
 
 #define LAUNCH(ctx, kernel, grid, block, smem, ...)                      \
@@ -736,7 +738,7 @@ extern "C" MSB_API int msb_state_destroy(msb_state *st) {
   for (size_t d = 0; d < st->D; d++) { cudaFree(st->d_niwW[d]); cudaFree(st->d_niwBias[d]); cudaFree(st->d_niwCoef[d]); cudaFree(st->d_niwB[d]); }
   cudaFree(st->d_niwA16);
   cudaFree(st->d_rowmax);
-  cudaFree(st->d_grid); cudaFree(st->d_hpwork); cudaFree(st->d_theta);
+  cudaFree(st->d_grid); cudaFree(st->d_hpwork); cudaFree(st->d_theta); cudaFree(st->d_hpsl);
   cudaFree(st->d_feats); cudaFree(st->d_feats_scalar); cudaFree(st->d_hp); cudaFree(st->d_ss); cudaFree(st->d_delta); cudaFree(st->d_delta_i32); cudaFree(st->d_counter);
   cudaFree(st->d_slot2gid); cudaFree(st->d_assign64); cudaFree(st->d_flags); cudaFreeHost(st->h_moved); cudaFreeHost(st->h_flags); cudaFree(st->d_assign); cudaFree(st->d_params); cudaFree(st->d_scores);
   cudaFree(st->d_base); cudaFree(st->d_base_score); cudaFree(st->d_col2slot); cudaFree(st->d_newslot); cudaFree(st->d_newcol); cudaFree(st->d_uniforms);
@@ -2960,6 +2962,164 @@ extern "C" MSB_API int msb_state_redraw_empty(msb_state *st, uint64_t seed, uint
     tf.push_back(t);
   }
   return theta_run(st, false, tf, seed, counter, nullptr);
+}
+
+// ---- slice sampling of continuous hypers (DESIGN.md section 4.12) ----------------------------------------------------
+// A spec's target, support and stream: msb_hpslice.cuh.  The feature index (alpha: D) is kept below 65535 like theta's.
+constexpr size_t HPSL_MAX_FEATURE = 65535;
+
+extern "C" MSB_API int msb_state_slice_hp(msb_state *st, const msb_slice_hp_opts *opts, msb_slice_hp_out *out) {
+  REQUIRE(st && opts, "NULL argument");
+  REQUIRE(opts->specs || opts->nspecs == 0, "NULL argument");
+  REQUIRE(opts->counter < (1ull << 32), "counter must be below 2^32");
+  if (out) out->capped = 0;
+  const size_t D = st->D, S = opts->nspecs;
+  std::vector<HpSliceFeat> tasks;
+  std::vector<std::vector<HpSliceSpec>> specs;     // per task, in the order given
+  std::vector<std::vector<size_t>> hp_offs;        // per task and spec: the key's offset in the feature's hp vector
+  std::map<size_t, size_t> task_of;
+  for (size_t i = 0; i < S; i++) {
+    const msb_slice_hp_spec &sp = opts->specs[i];
+    REQUIRE(sp.key, "NULL argument");
+    const size_t d = sp.feature;
+    const std::string key = sp.key;
+    REQUIRE(d <= D, "spec " + std::to_string(i) + ": feature index " + std::to_string(d) + " out of range (" + std::to_string(D) +
+                        " features; " + std::to_string(D) + " = alpha)");
+    const std::string who = d == D ? "alpha" : "feature " + std::to_string(d) + ": key '" + key + "'";
+    size_t off = 0, cnt = 1;
+    int slot = 0, partner = -1;
+    double lo = 0.0;
+    const msb_model_desc *m = d < D ? &st->models[d] : nullptr;
+    if (!m) {
+      if (key != "alpha") return fail(MSB_ERR_KEY, "alpha: unknown cluster hp key: " + key);
+    } else {
+      const int rc = hp_field(*m, key, &off, &cnt);
+      if (rc != MSB_OK) return fail(rc, "feature " + std::to_string(d) + ": " + g_last_error);
+      const bool vec = m->family == MSB_FAMILY_DD || m->family == MSB_FAMILY_DM ||
+                       (m->family == MSB_FAMILY_NIW && (key == "mu" || key == "psi"));
+      if (vec) return fail(MSB_ERR_UNSUPPORTED, who + ": a vector hyper cannot be slice-sampled; resample it on a grid (msb_state_set_hp_grid)");
+      REQUIRE(!(m->family == MSB_FAMILY_BNB && key == "r"),
+              who + ": bnb's score_data drops the r-dependent data term; only (alpha, beta) can be slice-sampled");
+      slot = (int)off;
+      if (m->family == MSB_FAMILY_NIW) {
+        slot = key == "kappa" ? 0 : 1;
+        if (key == "nu") lo = (double)m->dim - 1.0;
+      }
+      if (m->family == MSB_FAMILY_NICH && key == "mu") lo = -HUGE_VAL;
+    }
+    REQUIRE(d < HPSL_MAX_FEATURE, who + ": the feature index does not fit the stream packing (below 65535)");
+    REQUIRE(std::isfinite(sp.width) && sp.width > 0.0, who + ": the slice width must be finite and positive");
+    switch (sp.prior) {
+      case MSB_HPRIOR_FLAT:
+        REQUIRE(std::isfinite(sp.a) && std::isfinite(sp.b) && sp.a < sp.b, who + ": the flat prior needs finite lo < hi");
+        break;
+      case MSB_HPRIOR_EXPONENTIAL:
+        REQUIRE(std::isfinite(sp.a) && sp.a > 0.0, who + ": the exponential prior needs a finite rate > 0");
+        break;
+      case MSB_HPRIOR_NORMAL:
+        REQUIRE(std::isfinite(sp.a) && std::isfinite(sp.b) && sp.b > 0.0, who + ": the normal prior needs a finite mu and a finite s2 > 0");
+        break;
+      case MSB_HPRIOR_NONINFORMATIVE_BETA:
+        REQUIRE(m && (m->family == MSB_FAMILY_BB || m->family == MSB_FAMILY_BBNC || m->family == MSB_FAMILY_BNB) &&
+                    (key == "alpha" || key == "beta"),
+                who + ": the non-informative beta prior applies to the alpha and beta of bb, bbnc and bnb only");
+        partner = 1 - slot;
+        break;
+      default: return fail(MSB_ERR_INVALID, who + ": unknown prior kind " + std::to_string(sp.prior));
+    }
+    auto it = task_of.find(d);
+    if (it == task_of.end()) {
+      HpSliceFeat t;
+      memset(&t, 0, sizeof(t));
+      t.feat = (int32_t)d; t.niw = -1;
+      if (!m) {
+        t.h[0] = st->alpha;
+      } else {
+        const double *h = st->h_hp.data() + st->feats[d].hp_off;
+        if (m->family == MSB_FAMILY_NIW) { t.h[0] = h[m->dim]; t.h[1] = h[m->dim + 1 + (size_t)m->dim * m->dim]; }
+        else for (size_t j = 0; j < hp_size(*m); j++) t.h[j] = h[j];
+      }
+      it = task_of.emplace(d, tasks.size()).first;
+      tasks.push_back(t);
+      specs.emplace_back();
+      hp_offs.emplace_back();
+    }
+    for (const HpSliceSpec &o : specs[it->second]) REQUIRE(o.slot != slot, who + ": the key appears twice");
+    HpSliceSpec s;
+    memset(&s, 0, sizeof(s));
+    s.slot = slot; s.partner = partner; s.prior = sp.prior; s.out = (uint32_t)i;
+    s.w = sp.width; s.a = sp.a; s.b = sp.b; s.lo = lo;
+    specs[it->second].push_back(s);
+    hp_offs[it->second].push_back(off);
+  }
+  if (tasks.empty()) return MSB_OK;
+  msb_ctx *ctx = st->ctx;
+  CU_TRY(cudaSetDevice(ctx->device));
+  MSB_TRY(prepare_columns(st));
+  MSB_TRY(sync_small(st));
+  const size_t K = st->h_col2slot.size(), T = tasks.size();
+  std::vector<HpSliceSpec> flat;
+  size_t nniw = 0;
+  for (size_t i = 0; i < T; i++) {
+    tasks[i].first = (uint32_t)flat.size();
+    tasks[i].nspecs = (uint32_t)specs[i].size();
+    flat.insert(flat.end(), specs[i].begin(), specs[i].end());
+    if ((size_t)tasks[i].feat < D && st->feats[tasks[i].feat].kind == KIND_NIW) tasks[i].niw = (int32_t)nniw++;
+  }
+  // d_hpsl = [HpSliceFeat [T] | HpSliceSpec [S] | value [S] (fp64) | status [S] (u8) | pad | niw prep [nniw][K][3] | log |psi| [nniw]]
+  const size_t off_spec = sizeof(HpSliceFeat) * T, off_val = off_spec + sizeof(HpSliceSpec) * S, off_status = off_val + sizeof(double) * S,
+               off_prep = (off_status + S + 7) / 8 * 8, off_ld0 = off_prep + sizeof(double) * nniw * K * 3,
+               total = off_ld0 + sizeof(double) * nniw;
+  std::vector<char> h(off_val);
+  memcpy(h.data(), tasks.data(), off_spec);
+  memcpy(h.data() + off_spec, flat.data(), sizeof(HpSliceSpec) * S);
+  MSB_TRY(ensure(&st->d_hpsl, &st->hpsl_cap, total));
+  char *d = st->d_hpsl;
+  double *d_val = (double *)(d + off_val), *d_prep = (double *)(d + off_prep), *d_ld0 = (double *)(d + off_ld0);
+  uint8_t *d_status = (uint8_t *)(d + off_status);
+  CU_TRY(cudaMemcpyAsync(d, h.data(), h.size(), cudaMemcpyHostToDevice, ctx->stream));  // pageable: staged on return
+  CU_TRY(cudaMemsetAsync(d_status, 0xff, S, ctx->stream));
+  for (const HpSliceFeat &t : tasks) {
+    if (t.niw < 0) continue;
+    const FeatDev &f = st->feats[t.feat];
+    const size_t smem = ((size_t)f.dim * f.dim + f.dim) * sizeof(double);
+    if (smem > 48 * 1024) CU_TRY(opt_in_smem(niw_slice_prep_kernel, smem));
+    LAUNCH(ctx, niw_slice_prep_kernel, (unsigned)(K + 1), 128, smem, f, st->d_hp, st->d_ss, st->d_col2slot, (int)K,
+           d_prep + (size_t)t.niw * K * 3, d_ld0 + t.niw);
+  }
+  LAUNCH(ctx, hp_slice_kernel, (unsigned)T, HP_THREADS, 0, st->d_feats, (int)D, (const HpSliceFeat *)d,
+         (const HpSliceSpec *)(d + off_spec), st->d_ss, st->d_col2slot, (int)K, d_prep, d_ld0, opts->seed, opts->counter, d_val,
+         d_status);
+  std::vector<char> r(off_status + S - off_val);
+  CU_TRY(cudaMemcpyAsync(r.data(), d_val, r.size(), cudaMemcpyDeviceToHost, ctx->stream));
+  CU_TRY(cudaStreamSynchronize(ctx->stream));
+  const double *val = (const double *)r.data();
+  const uint8_t *status = (const uint8_t *)(r.data() + sizeof(double) * S);
+  for (size_t i = 0; i < S; i++)
+    if (status[i] == HPSL_BAD) {
+      const msb_slice_hp_spec &sp = opts->specs[i];
+      return fail(MSB_ERR_INVALID, (sp.feature == D ? std::string("alpha") : "feature " + std::to_string(sp.feature) + ": key '" + sp.key + "'") +
+                                       ": the target (log prior + score_data) is not finite at the current value; the slice update needs a finite density there");
+    }
+  size_t capped = 0;
+  for (size_t i = 0; i < T; i++) {
+    const size_t f = tasks[i].feat;
+    if (f == D) { st->alpha = val[specs[i][0].out]; continue; }
+    std::vector<double> v(st->h_hp.begin() + st->feats[f].hp_off, st->h_hp.begin() + st->feats[f].hp_off + hp_size(st->models[f]));
+    bool changed = false;
+    for (size_t j = 0; j < specs[i].size(); j++) {
+      const double x = val[specs[i][j].out];
+      changed |= memcmp(&x, &v[hp_offs[i][j]], sizeof(double)) != 0;
+      v[hp_offs[i][j]] = x;
+    }
+    if (changed) write_hp(st, f, 0, v.data(), v.size());
+  }
+  for (size_t i = 0; i < S; i++) {
+    capped += status[i] == HPSL_CAPPED;
+    if (out && out->values) out->values[i] = val[i];
+  }
+  if (out) out->capped = capped;
+  return MSB_OK;
 }
 
 // ---- one pass over host rows in ONE call ---------------------------------------------------------------------------

@@ -23,6 +23,21 @@ def flat_hp(model, hp):
     return np.concatenate([np.asarray(hp[k], np.float64).ravel() for k in model.default_hyperparams()])
 
 
+def slice_hp_specs(hparams, cparam, nfeatures):
+    """the msb_slice_hp_spec list of state.slice_hp: (feature, key, width, prior kind, a, b) per update, the features in
+    the order given, each feature's keys in its dict's order with a tuple key expanded in place, then alpha as feature
+    ``nfeatures``"""
+    specs = []
+    items = list((hparams or {}).items()) + [(nfeatures, {k: v}) for k, v in (cparam or {}).items()]
+    for d, params in items:
+        for key, (prior, width) in params.items():
+            if not hasattr(prior, "kind"):
+                raise TypeError("component %r, key %r: the prior must be one of common_b200.hyperprior's" % (d, key))
+            for k in (key if isinstance(key, tuple) else (key,)):
+                specs.append((int(d), k, float(width), int(prior.kind), prior.a, prior.b))
+    return specs
+
+
 class state(object):
     def __init__(self, ctx, models, max_groups=64, cluster_hp=None):
         self._ctx = ctx
@@ -157,6 +172,29 @@ class state(object):
     def redraw_empty(self, seed=0, counter=0):
         """every empty group's bbnc p drawn afresh from Beta(alpha, beta): the auxiliary groups of Neal's algorithm 8"""
         _lib.check(_lib.load().msb_state_redraw_empty(self._h, int(seed), int(counter)))
+
+    # ---- slice sampling of continuous hypers (msb_state_slice_hp) ------------------------------------------------
+    def slice_hp(self, hparams=None, cparam=None, seed=0, counter=0):
+        """one slice-sampling update of every listed scalar hyper, on the device and applied to the state.
+        ``hparams`` is the runner's {component: {key: (prior, width)}}, ``cparam`` {"alpha": (prior, width)}, with the
+        priors of common_b200.hyperprior; a tuple key such as ("alpha", "beta") gives one update per key, in that order.
+        Returns {"capped": updates that reached the shrink cap, "values": {component: {key: value}, "alpha": value}}"""
+        specs = slice_hp_specs(hparams, cparam, len(self._models))
+        arr = (_lib.SliceHpSpec * max(len(specs), 1))()
+        keys = [key.encode() for _, key, _, _, _, _ in specs]       # kept alive for the call
+        for i, (d, _, w, kind, a, b) in enumerate(specs):
+            arr[i] = _lib.SliceHpSpec(d, keys[i], w, kind, a, b)
+        values = np.zeros(max(len(specs), 1))
+        out = _lib.SliceHpOut(0, values.ctypes.data)
+        opts = _lib.SliceHpOpts(int(seed), int(counter), arr, len(specs))
+        _lib.check(_lib.load().msb_state_slice_hp(self._h, C.byref(opts), C.byref(out)))
+        res = {}
+        for i, (d, key, _, _, _, _) in enumerate(specs):
+            if d == len(self._models):
+                res["alpha"] = float(values[i])
+            else:
+                res.setdefault(d, {})[key] = float(values[i])
+        return {"capped": out.capped, "values": res}
 
     # ---- suffstats (entity_state.hpp:51-54) --------------------------------------
     def get_suffstats(self, component, gid, key, count=1):

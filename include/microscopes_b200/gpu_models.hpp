@@ -357,6 +357,18 @@ public:
   }
   // every empty group's bbnc p drawn afresh from Beta(alpha, beta) (msb_state_redraw_empty)
   void redraw_empty(uint64_t seed, uint64_t counter) { b200::check(msb_state_redraw_empty(st_, seed, counter)); }
+  // one slice-sampling update per spec of scalar feature hypers and of alpha (feature D), applied to the state
+  // (msb_state_slice_hp); returns each spec's value after the call, and the number that reached the shrink cap in *capped
+  std::vector<double> slice_hp(const std::vector<msb_slice_hp_spec> &specs, uint64_t seed, uint64_t counter, size_t *capped = nullptr) {
+    std::vector<double> values(specs.size());
+    msb_slice_hp_opts o;
+    o.seed = seed; o.counter = counter; o.specs = specs.data(); o.nspecs = specs.size();
+    msb_slice_hp_out out;
+    out.capped = 0; out.values = values.data();
+    b200::check(msb_state_slice_hp(st_, &o, &out));
+    if (capped) *capped = out.capped;
+    return values;
+  }
   msb_sweep_result sweep(uint64_t seed, uint64_t sweep_id) {
     msb_sweep_opts o;
     std::memset(&o, 0, sizeof(o));

@@ -33,6 +33,7 @@
  *   msb_state_theta / redraw_empty
  *                         mixturemodel's theta kernel (slice sampling of bbnc's p) and the auxiliary-parameter
  *                         step of its assign_resample kernel (Neal's algorithm 8: the empty groups' p from the prior)
+ *   msb_state_slice_hp    mixturemodel's slice hp kernel: one slice update of scalar feature hypers and of alpha
  *   msb_value_*           single-value group::score_value/add_value/remove_value/score_data/sample_value
  *                         (models/base.hpp:25-27), executed on the device
  *
@@ -320,7 +321,7 @@ MSB_API int msb_state_predict(msb_state *st, size_t row_lo, size_t row_hi, const
 
 /* ---- hyperparameter inference on a grid (DESIGN.md section 4.10) -----------------------------------------------------
  * The mixturemodel runner's grid feature-hp kernel and its cluster-hp kernel, on the device.  Grids are registered once
- * and stay resident; the caller supplies the log hyperprior of every point (the library evaluates no hyperprior density).
+ * and stay resident; the caller supplies the log hyperprior of every point (msb_state_slice_hp, below, evaluates its own).
  *
  * msb_state_set_hp_grid: feature `feature` gets npoints >= 1 grid points, each a complete hp vector in the flat layout
  * msb_value_score_data takes (nhp doubles; bb: alpha, beta; bnb: alpha, beta, r; gp: alpha, inv_beta; nich: mu, kappa,
@@ -380,6 +381,54 @@ typedef struct msb_theta_opts {
 typedef struct msb_theta_out { size_t capped; } msb_theta_out;
 MSB_API int msb_state_theta(msb_state *st, const msb_theta_opts *opts, msb_theta_out *out);
 MSB_API int msb_state_redraw_empty(msb_state *st, uint64_t seed, uint64_t counter);
+
+/* ---- slice sampling of continuous hypers (DESIGN.md section 4.12) ----------------------------------------------------
+ * msb_state_slice_hp: the mixturemodel runner's slice hp kernel.  Each spec gets one univariate slice update (Neal 2003)
+ * of one scalar hyper of one feature, or of the CRP concentration (feature == D, key "alpha").  The target is
+ *   f(x) = log prior(x) + sum over every group column (ascending gid, empty groups included) of score_data with x
+ *          substituted -- fp64, the set msb_state_hp_gibbs sums, with its fixed order and no atomics;
+ *   alpha: log prior(x) + (#non-empty groups - 1) log x + lgamma(1 + x) - lgamma(n + x), n = assigned entities;
+ * and -inf outside the key's support.  Sliceable keys and supports: bb, bbnc, bnb alpha, beta (0, inf) -- bbnc's given
+ * the groups' p; gp alpha, inv_beta (0, inf); nich mu (real line), kappa, sigmasq, nu (0, inf); niw(d) kappa (0, inf),
+ * nu (d - 1, inf); alpha (0, inf).
+ * The update: y = f(x0) + log u; L = x0 - w u', R = L + w; bounded stepping out with m = 128 (L at most floor(m V)
+ * times, R at most m - 1 - floor(m V) times, while f > y); then shrinkage, at most 200 steps.  A spec that reaches the cap
+ * keeps x0 and is counted in out->capped.  A feature's specs run in the order given, each conditioning on the values its
+ * predecessors drew; features and alpha are independent given the partition.  Spec j (its index among its feature's
+ * specs) of feature d reads philox4x32_10(key = seed, counter = (counter << 32 | d, HPSL_TAG | j << 16 | block)),
+ * HPSL_TAG = "HPSL" << 32: identical suffstats and hypers give identical values, on every replica.
+ * After the call's one synchronise, and only if nothing was refused, every changed feature's hp vector is written as
+ * msb_state_set_hp writes it and alpha as msb_state_set_cluster_hp does; assignments, suffstats, deltas and the sweep
+ * timing ring do not change.  Pending deferred deltas are not included.
+ * Refused, the state untouched, with MSB_ERR_KEY for a key the family does not have, MSB_ERR_UNSUPPORTED for a vector
+ * key (dd / dm alphas, niw mu / psi: resample them on a grid with msb_state_set_hp_grid), and MSB_ERR_INVALID (the
+ * message names the feature and the key) for: bnb's r (score_data drops its data term), a width <= 0 or not finite,
+ * prior parameters outside the ranges below, the non-informative prior on anything but the alpha / beta of bb, bbnc or
+ * bnb, a key twice for one feature, a feature index > D or >= 65535, counter >= 2^32, a current value where f is not
+ * finite (e.g. outside the flat prior's interval, niw nu <= d - 1, a bbnc group whose p is 0 while it has heads), and
+ * no groups. */
+enum msb_hprior {                       /* the reference's in-tree hyperpriors, plus a flat interval */
+  MSB_HPRIOR_FLAT = 0,                  /* a = lo, b = hi:      0 on (lo, hi), -inf outside; lo < hi, both finite */
+  MSB_HPRIOR_EXPONENTIAL = 1,           /* a = rate > 0:        log(rate) - rate x for x >= 0, -inf below (log_exponential) */
+  MSB_HPRIOR_NORMAL = 2,                /* a = mu, b = s2 > 0:  -0.5 log(2 pi s2) - (x - mu)^2 / (2 s2)   (log_normal) */
+  MSB_HPRIOR_NONINFORMATIVE_BETA = 3    /* -2.5 log(alpha + beta), the partner at its current value (log_noninformative_beta_prior) */
+};
+typedef struct msb_slice_hp_spec {
+  size_t feature;                       /* < D, or D for the CRP concentration (key "alpha") */
+  const char *key;                      /* a scalar hp key of the family, as msb_state_set_hp names it */
+  double width;                         /* slice width w > 0 */
+  int32_t prior;                        /* enum msb_hprior */
+  double a, b;                          /* the prior's parameters */
+} msb_slice_hp_spec;
+typedef struct msb_slice_hp_opts {
+  uint64_t seed, counter;
+  const msb_slice_hp_spec *specs; size_t nspecs;
+} msb_slice_hp_opts;
+typedef struct msb_slice_hp_out {
+  size_t capped;                        /* specs that reached the shrink cap and kept their value */
+  double *values;                       /* [nspecs] or NULL: each spec's value after the call */
+} msb_slice_hp_out;
+MSB_API int msb_state_slice_hp(msb_state *st, const msb_slice_hp_opts *opts, msb_slice_hp_out *out);
 
 /* multi-GPU: flat fp64 buffer [group counts | per-feature suffstat deltas] on the device */
 MSB_API int msb_state_delta_buffer(msb_state *st, double **dev_ptr, size_t *count);
